@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- queries/sec of exact tree inference (BASELINE.json metric) on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic range-predicate queries:
@@ -69,7 +69,26 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--streams", type=int, default=2, help="launch consecutive (independent) steps on this many streams in turn")
     ap.add_argument("--inproc", action="store_true", help="add the in-process multi-GPU leg (one process, all visible GPUs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the probabilities of the last timed step (rank 0) to DIR/probabilities.npy, float32")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is available for --impl ours only")
+    return args
+
+
+DUMP_MAX_VALUES = 15_000_000   # 60 MB of float32: larger batches are dumped as a fixed, seeded sample
+
+
+def dump_outputs(out_dir, probs):
+    """Write the results a caller of the timed path receives, so that two builds can be compared value for value."""
+    probs = np.asarray(probs, dtype=np.float32)
+    if probs.size > DUMP_MAX_VALUES:
+        probs = probs[np.sort(np.random.default_rng(SEED).choice(probs.size, DUMP_MAX_VALUES, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "probabilities.npy"), probs)
 
 
 def load_tree(name):
@@ -660,6 +679,8 @@ def run_ours(args):
     launches = launch_count() - launches0
     ms = max_over_ranks(e0.elapsed_time(e1))
     value = world * B * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:   # copied now: the legs below reuse the result buffers
+        dump_outputs(args.dump_outputs, outs[(args.steps - 1) % n_streams].cpu().numpy())
 
     # ---- sustained: the same launch back to back for >= sustained_seconds ----------------------------
     sustained = None
