@@ -118,6 +118,10 @@ _SIGS = {
                                   C.c_void_p, C.POINTER(C.c_size_t)]),
     "bc_fit_counts": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_size_t,
                                 C.c_void_p, C.c_size_t, C.POINTER(C.c_uint32), C.c_void_p]),
+    "bc_pair_counts": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_size_t, C.c_void_p,
+                                 C.c_size_t, C.POINTER(C.c_uint32), C.c_void_p]),
+    "bc_chow_liu": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_void_p,
+                              C.c_size_t, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32), C.c_void_p]),
     "bc_measure_fp32_peak": (C.c_int, [C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "bc_launch_count": (C.c_uint64, []),
     "bc_last_error": (C.c_char_p, []),

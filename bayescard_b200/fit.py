@@ -6,7 +6,7 @@ node the 2-D histogram of (own bin, parent bin), an all-zero column replaced by 
 histogram pass is one CUDA kernel over the discretised table (``bc_fit_counts``, ``csrc/bc_fit.cu``); the few thousand
 fp64 divisions happen here, written the way the reference writes them so that the CPTs are bit-identical.
 
-Structure learning (pomegranate's Chow-Liu) stays out of scope: the tree is an input.
+The tree is an input here; :mod:`.structure` learns it (pomegranate's Chow-Liu) from the same kind of table.
 """
 from __future__ import annotations
 

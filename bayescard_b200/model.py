@@ -58,6 +58,16 @@ class Bayescard_BN:
         """Load a reference pickle (``pickle.dump(Bayescard_BN)``) or the flat ``.npz`` form."""
         return cls(load_model(path), device=device, **kw)
 
+    @classmethod
+    def build_from_table(cls, table, card, names=None, root=0, device=0, table_name="table", **kw) -> "Bayescard_BN":
+        """Table-level counterpart of the reference's ``build_from_data`` (without its discretisation): learn the Chow-Liu
+        tree of a table of bin ids (``[n_rows, n_cols]`` uint8 / uint16) and fit its CPTs on the GPU
+        (:func:`.structure.learn_tree_model`).  The result is ready for ``init_inference_method()``."""
+        from .structure import learn_tree_model
+
+        return cls(learn_tree_model(table, card, names=names, root=root, device=device, table_name=table_name),
+                   device=device, **kw)
+
     def __str__(self):
         return f"bn{self.table_name}.{self.algorithm}-{self.max_parents}-{self.root}-{self.n_mcv}-{self.n_bins}"
 

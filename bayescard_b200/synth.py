@@ -65,3 +65,25 @@ def pack_ranges_u16(lo: np.ndarray, hi: np.ndarray) -> np.ndarray:
     out[:, 0::2] = lo
     out[:, 1::2] = hi
     return out
+
+
+def sample_table_device(tm: TreeModel, n: int, seed: int = 0, device: int = 0):
+    """Ancestral sample of ``n`` rows of ``tm`` on the device: a ``[n, n_nodes]`` uint8 (uint16 when a card exceeds
+    256) torch tensor, columns in the model's topological order.  torch is plumbing here (seeded ``torch.rand``)."""
+    import torch
+
+    dev = torch.device("cuda", device)
+    dtype = torch.uint8 if int(np.max(tm.card)) <= 256 else torch.int16
+    g = torch.Generator(device=dev).manual_seed(seed)
+    cols = []
+    for v in range(tm.n_nodes):
+        pa = int(tm.parent[v])
+        t = torch.tensor(np.asarray(tm.cpts[v], dtype=np.float64).reshape(int(tm.card[v]), -1), device=dev)
+        cdf = torch.cumsum(t / t.sum(dim=0, keepdim=True), dim=0).T.contiguous()   # [card_pa, card]
+        u = torch.rand(n, generator=g, device=dev, dtype=torch.float64)
+        idx = cols[pa].long() if pa >= 0 else torch.zeros(n, dtype=torch.long, device=dev)
+        out = torch.empty(n, dtype=torch.long, device=dev)
+        for s in range(0, n, 1 << 22):   # bounded [rows, card] temporaries
+            out[s:s + (1 << 22)] = (cdf[idx[s:s + (1 << 22)]] < u[s:s + (1 << 22), None]).sum(dim=1)
+        cols.append(torch.clamp(out, max=int(tm.card[v]) - 1).to(dtype))
+    return torch.stack(cols, dim=1).contiguous()

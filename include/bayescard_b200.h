@@ -309,6 +309,35 @@ BC_API int bc_fit_counts(int device, int n_nodes, const int32_t* parent, const i
                          int elem_bytes, size_t n_rows, size_t row_stride_elems, unsigned long long* counts_dev,
                          size_t n_counters, uint32_t* bad_rows_host, void* stream);
 
+/* ---- Structure learning: all-pairs counts, mutual information, Chow-Liu tree ------------------------------------
+ * Replaces pomegranate's BayesianNetwork.from_samples(algorithm='chow-liu', root=0) (Models/BN_single_model.py:141-202).
+ *   table_dev   DEVICE pointer, n_rows rows of bin ids, row-major, columns in ANY order, elem_bytes 1 (uint8) or 2
+ *               (uint16), row stride row_stride_elems (>= n_cols) elements; n_cols >= 2; 1 <= card[i] <= 256 (uint8)
+ *               or 65536 (uint16); sum of the cards, padded to a multiple of 256, at most 16384 (BC_ELIMIT beyond)
+ *   counts_dev  DEVICE pointer to n_counters + 1 64-bit counters, zeroed by the call.  Layout: per column i its
+ *               marginal counts (card[i] counters, at C_i = sum_{k<i} card[k]); then for every pair i < j in
+ *               row-major pair order (0,1), (0,2), ..., (1,2), ... the block card[i] x card[j], row-major ([a][b] =
+ *               rows with bin a in column i and bin b in column j); then ONE extra counter, the number of skipped rows
+ *   bad_rows_host  (nullable) rows skipped because a bin id was >= its column's card (a skipped row counts nowhere,
+ *               as in bc_fit_counts); reading it synchronises the stream
+ * The counting is one int8 tensor-core GEMM (one-hot(table)^T . one-hot(table)) with s32 accumulation: exact. */
+BC_API int bc_pair_counts(int device, int n_cols, const int32_t* card, const void* table_dev, int elem_bytes, size_t n_rows,
+                          size_t row_stride_elems, unsigned long long* counts_dev, size_t n_counters,
+                          uint32_t* bad_rows_host, void* stream);
+/* The Chow-Liu tree of the table: bc_pair_counts, then MI[i][j] = sum_ab (n_ab/N) log(N n_ab / (n_a n_b)) over
+ * n_ab > 0 in fp64 on the device (N = rows kept; pomegranate's mutual information with pseudocount 0, scaled by N),
+ * then Prim's maximum spanning tree on the host, rooted at `root`.  Tie rule (pomegranate's discrete_chow_liu_tree):
+ * the next edge is the (in-tree x, outside y) pair of largest MI, x scanned in the order the nodes joined, y
+ * ascending, only a strictly larger MI replacing the best so far.
+ *   parent_host  int32[n_cols]: parent column of every column, -1 for the root (table column order)
+ *   counts_dev   (nullable) receives the counts as bc_pair_counts writes them (n_counters + 1 counters); when NULL
+ *                the counts live in a temporary buffer and n_counters is ignored
+ *   mi_host      (nullable) fp64[n_cols * n_cols], symmetric, zero diagonal
+ * Synchronous: returns when the tree is known. */
+BC_API int bc_chow_liu(int device, int n_cols, const int32_t* card, const void* table_dev, int elem_bytes, size_t n_rows,
+                       size_t row_stride_elems, int root, unsigned long long* counts_dev, size_t n_counters,
+                       int32_t* parent_host, double* mi_host, uint32_t* bad_rows_host, void* stream);
+
 /* Measured FP32 FFMA peak of the device (TFLOP/s), the roofline denominator SURVEY.md section 8d
  * asks to measure in the same run rather than quote. */
 BC_API int bc_measure_fp32_peak(int device, double* tflops, double* sm_clock_mhz);

@@ -5,10 +5,8 @@ copied from a random earlier column, range / equality queries with known true ca
 where the reference's discretiser (``Models/tools.py:49-128`` with ``n_mcv=30, n_bins=70``) keeps every value as its own
 bin, so the states ARE the values.
 
-Per configuration: generate the table (cell 1 ``data_generation``), learn a Chow-Liu tree (maximum spanning tree on
-pairwise mutual information, rooted at column 0 -- what ``pomegranate`` does for the reference; structure learning is not
-part of the hot path, this is a tool), fit the CPTs on the GPU (``bayescard_b200.fit``, the reference's pgmpy MLE
-counts), draw the queries (cell 1 ``generate_single_query``), evaluate them through the drop-in ``Bayescard_BN.query``
+Per configuration: generate the table (cell 1 ``data_generation``), learn the Chow-Liu tree rooted at column 0 and its
+CPTs on the GPU (``bayescard_b200.structure.learn_tree_model``, what ``pomegranate`` + pgmpy do for the reference), draw the queries (cell 1 ``generate_single_query``), evaluate them through the drop-in ``Bayescard_BN.query``
 (scalar latency, as the notebook times it) and ``query_batch``, and print the q-error percentiles and latency beside
 the paper's Table 11 rows.
 
@@ -61,52 +59,6 @@ def data_generation(rng, skew, domain_size, correlation, column_size, nrows):
     return data.T.astype(np.int64)   # [nrows, column_size]
 
 
-def chow_liu_tree(table, card, sample=20000, seed=0):
-    """Maximum spanning tree on pairwise mutual information (Prim), rooted at column 0: parent[v] in table column order."""
-    rng = np.random.default_rng(seed)
-    rows = table[rng.choice(table.shape[0], size=min(sample, table.shape[0]), replace=False)]
-    n = table.shape[1]
-    mi = np.zeros((n, n))
-    for a in range(n):
-        for b in range(a + 1, n):
-            joint = np.zeros((card, card))
-            np.add.at(joint, (rows[:, a], rows[:, b]), 1.0)
-            joint /= joint.sum()
-            pa, pb = joint.sum(1, keepdims=True), joint.sum(0, keepdims=True)
-            nz = joint > 0
-            mi[a, b] = mi[b, a] = float((joint[nz] * np.log(joint[nz] / (pa @ pb)[nz])).sum())
-    parent = np.full(n, -1, dtype=np.int64)
-    in_tree = np.zeros(n, dtype=bool)
-    in_tree[0] = True
-    best = mi[0].copy()
-    link = np.zeros(n, dtype=np.int64)
-    for _ in range(n - 1):
-        cand = np.where(in_tree, -np.inf, best)
-        v = int(np.argmax(cand))
-        parent[v] = link[v]
-        in_tree[v] = True
-        upd = (~in_tree) & (mi[v] > best)
-        best[upd] = mi[v][upd]
-        link[upd] = v
-    return parent
-
-
-def topological(parent):
-    """Order with parents before children (root first); returns (order, parent in the new numbering)."""
-    n = len(parent)
-    kids = [[] for _ in range(n)]
-    for v, p in enumerate(parent):
-        if p >= 0:
-            kids[p].append(v)
-    order, stack = [], [0]
-    while stack:
-        v = stack.pop()
-        order.append(v)
-        stack.extend(reversed(kids[v]))
-    pos = {v: i for i, v in enumerate(order)}
-    return order, np.asarray([-1 if parent[v] < 0 else pos[parent[v]] for v in order], dtype=np.int32)
-
-
 def generate_queries(rng, table, card, num, p=0.8, nval=4, skip_zero_bit=4):
     """Cell 1 ``generate_single_query``: (lo, hi) per column (full domain when unpredicated) + the true cardinality."""
     nrows, n = table.shape
@@ -141,9 +93,8 @@ def q_errors(pred, true):
 
 def run_one(skew, domain, corr, ncols, nrows, nq, seed, device=0, p=0.8, skip_zero_bit=4):
     from bayescard_b200 import _lib as L
-    from bayescard_b200 import fit
     from bayescard_b200.engine import DeviceModel
-    from bayescard_b200.loader import TreeModel
+    from bayescard_b200.structure import learn_tree_model
     from bayescard_b200.synth import pack_ranges_u16
 
     rng = np.random.default_rng(seed)
@@ -151,18 +102,12 @@ def run_one(skew, domain, corr, ncols, nrows, nq, seed, device=0, p=0.8, skip_ze
     table = data_generation(rng, skew, domain, corr, ncols, nrows)
     t_gen = time.perf_counter() - t0
     t0 = time.perf_counter()
-    order, parent = topological(chow_liu_tree(table, domain, seed=seed))
-    t_struct = time.perf_counter() - t0
-    table_t = np.ascontiguousarray(table[:, order].astype(np.uint8))
+    names = [f"attr{c}" for c in range(ncols)]
     card = np.full(ncols, domain, dtype=np.int32)
-    t0 = time.perf_counter()
-    cpts, _, bad = fit.fit_cpts(parent, card, table_t, device)
-    t_fit = time.perf_counter() - t0
-    assert bad == 0
-    names = [f"attr{v}" for v in order]
-    tm = TreeModel(table_name="toy", nrows=nrows, node_names=names, structure=tuple(() if p < 0 else (int(p),) for p in parent),
-                   attr_type={k: "categorical" for k in names}, algorithm="chow-liu", topo_names=names, infer_names=names,
-                   parent=parent, card=card, cpts=cpts, dropped_names=[])
+    tm = learn_tree_model(table.astype(np.uint8), card, names=names, root=0, device=device, table_name="toy")
+    t_struct = time.perf_counter() - t0   # tree and CPTs: one pass over the table on the GPU
+    order = [names.index(x) for x in tm.infer_names]
+    table_t = np.ascontiguousarray(table[:, order].astype(np.uint8))
     lo, hi, true = generate_queries(rng, table_t.astype(np.int64), domain, nq, p=p, skip_zero_bit=skip_zero_bit)
     dm = DeviceModel(tm, device=device, specialize=ncols * domain * domain <= 200_000)   # (the straight-line kernel is for small models)
     desc = pack_ranges_u16(lo.astype(np.int32), hi.astype(np.int32))
@@ -179,7 +124,7 @@ def run_one(skew, domain, corr, ncols, nrows, nq, seed, device=0, p=0.8, skip_ze
     return {"skew": skew, "domain": domain, "correlation": corr, "columns": ncols, "rows": nrows, "queries": nq, "p": p, "skip_zero_bit": skip_zero_bit,
             "q_error_50_90_95_99_100": [float(np.percentile(qe, x)) for x in (50, 90, 95, 99, 100)],
             "latency_ms_scalar_p50": float(np.median(lat[5:]) * 1e3), "latency_ms_scalar_mean": float(np.mean(lat[5:]) * 1e3),
-            "batch_ms": t_batch * 1e3, "seconds": {"generate": t_gen, "chow_liu": t_struct, "fit_gpu": t_fit}}
+            "batch_ms": t_batch * 1e3, "seconds": {"generate": t_gen, "chow_liu_and_fit_gpu": t_struct}}
 
 
 def main():
