@@ -253,6 +253,7 @@ extern "C" void bc_model_destroy(bc_model* m) {
         bc_k2_free(m);
         bc_k3_free(m);
         if (m->spec_lib) cudaLibraryUnload(m->spec_lib);
+        bc_marg_free(m);
         cudaFree(m->d_arena);
         cudaFree(m->d_fan);
         cudaFree(m->d_nodes);

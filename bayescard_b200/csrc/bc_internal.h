@@ -16,6 +16,7 @@
 #define BC_VERSION_STRING "bayescard_b200 0.1.0 (sm_100a)"
 #define BC_CODEGEN_VERSION 10
 #define BC_SPEC_CTR_SLOTS 256
+#define BC_MARGINAL_VERSION 1   // marginal kernels (bc_marg_*): part of their cache name, independent of BC_CODEGEN_VERSION
 
 // One record per node, copied to the device and (by K1) into shared memory.  32 bytes.
 struct BcNodeRec {
@@ -32,6 +33,14 @@ struct BcNodeRec {
 struct BcBitsRec {
     int32_t bit_off;     // first bit of this node's state mask in a BITS row
     int32_t card;
+};
+
+// Specialised marginal kernels of one target node (spec_jit.cu)
+struct BcMargSlot {
+    cudaLibrary_t lib = nullptr;
+    cudaKernel_t bits = nullptr, dense = nullptr;
+    int threads = 0;
+    int blocks_bits = 1, blocks_dense = 1;   // resident CTAs per SM
 };
 
 struct BcHostPipe;  // bc_api.cu
@@ -88,6 +97,9 @@ struct bc_model {
     // leaves its slot zeroed
     uint64_t* d_spec_ctr = nullptr;
     std::atomic<uint32_t> spec_ctr_next{0};
+    // specialised marginal kernels, one slot per target node (empty until the first bc_model_specialize_marginal)
+    std::vector<BcMargSlot> marg;
+    std::mutex marg_mu;
     BcK2Plan* k2 = nullptr;
     std::mutex k2_mu;                // guards the lazy construction of k2 (pipe_mu may already be held)
     BcK3Plan* k3 = nullptr;          // fused tensor-core tree kernel: edge schedule, TMEM columns, operand images
@@ -144,3 +156,10 @@ int bc_spec_launch(bc_model* m, const void* desc, size_t nq, int fmt, const uint
                    float* out, cudaStream_t stream);
 int bc_spec_attach(bc_model* m, const void* image, size_t bytes);
 int bc_spec_build(bc_model* m, const char* cache_dir);
+// marginal kernels: spec_codegen.cc (source, hash) and spec_jit.cu (attach, launch)
+std::string bc_marginal_generate(const bc_model& m, int target);
+uint64_t bc_marginal_hash_of(const bc_model& m, int target);
+int bc_marg_build(bc_model* m, int target, const char* cache_dir);
+bool bc_marg_attached(bc_model* m, int target);
+int bc_marg_launch(bc_model* m, const void* desc, size_t nq, int fmt, int target, float* out, cudaStream_t stream);
+void bc_marg_free(bc_model* m);

@@ -1,0 +1,136 @@
+// GROUP BY on one column: out[q][b] = sum_{x : x_t = b} prod_v w_v[x_v] T_v[x_v, x_pa(v)] for every state b of a target node t.
+//
+// Two paths (see include/bayescard_b200.h, bc_marginal_batch):
+//   - the specialised marginal kernel of (model, t) (spec_codegen.cc / spec_jit.cu): one upward pass plus one downward
+//     chain along the root -> t path per query, card(t) results per thread;
+//   - the expansion, for every model the existing kernels serve: each row becomes card(t) rows, row b with the target's
+//     weights restricted to state b, evaluated q-major by bc_query_batch, so its results already are out[q][b].
+#include <cstring>
+
+#include "bc_internal.h"
+
+namespace {
+
+// BITS: row (q, b) = row q with the target's bits [off, off + card) ANDed with the one-hot of bit off + b.
+__global__ void expand_bits_kernel(const uint32_t* __restrict__ src, uint32_t* __restrict__ dst, size_t nq, int words, int card,
+                                   int off) {
+    const size_t total = nq * (size_t)card * words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const int w = (int)(i % words);
+        const size_t r = i / words;
+        const size_t q = r / card;
+        const int b = (int)(r % card);
+        uint32_t x = src[q * words + w];
+        const int lo = w * 32, hi = lo + 32;   // bits of this word: [lo, hi)
+        const int a = off > lo ? off : lo, e = off + card < hi ? off + card : hi;
+        if (a < e) {
+            const uint32_t tmask = (uint32_t)((((uint64_t)1 << (e - a)) - 1) << (a - lo));
+            const int bit = off + b;
+            const uint32_t keep = (bit >= lo && bit < hi) ? 1u << (bit - lo) : 0u;
+            x &= ~tmask | keep;
+        }
+        dst[i] = x;
+    }
+}
+
+// DENSE_F32: row (q, b) = row q with every weight of the target except state b set to 0.
+__global__ void expand_dense_kernel(const float* __restrict__ src, float* __restrict__ dst, size_t nq, int width, int card, int off) {
+    const size_t total = nq * (size_t)card * width;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const int j = (int)(i % width);
+        const size_t r = i / width;
+        const size_t q = r / card;
+        const int b = (int)(r % card);
+        float x = src[q * width + j];
+        if (j >= off && j < off + card && j != off + b) x = 0.f;
+        dst[i] = x;
+    }
+}
+
+constexpr size_t kExpandBytes = 256u << 20;   // bound on the expanded rows of one chunk
+
+int expand_path(bc_model* m, const void* desc, size_t nq, int fmt, int target, float* out, int kernel, cudaStream_t st) {
+    const int card = m->nodes[target].card;
+    const size_t stride = (size_t)bc_model_desc_stride(m, fmt);
+    const size_t row_bytes = stride * card;   // expanded bytes per query
+    size_t chunk = kExpandBytes / row_bytes;
+    if (chunk < 1) chunk = 1;
+    if (chunk > nq) chunk = nq;
+    void* scratch = nullptr;
+    BC_CUDA_CHECK(cudaMallocAsync(&scratch, chunk * row_bytes, st));
+    const int threads = 256;
+    int rc = BC_OK;
+    for (size_t q0 = 0; q0 < nq && rc == BC_OK; q0 += chunk) {
+        const size_t cq = nq - q0 < chunk ? nq - q0 : chunk;
+        const size_t elems = cq * row_bytes / 4;
+        long long grid = (long long)((elems + threads - 1) / threads);
+        if (grid > (long long)m->sm_count * 16) grid = (long long)m->sm_count * 16;
+        const unsigned char* src = static_cast<const unsigned char*>(desc) + q0 * stride;
+        if (fmt == BC_DESC_BITS)
+            expand_bits_kernel<<<(unsigned)grid, threads, 0, st>>>(reinterpret_cast<const uint32_t*>(src), static_cast<uint32_t*>(scratch),
+                                                                   cq, (int)(stride / 4), card, m->bits[target].bit_off);
+        else
+            expand_dense_kernel<<<(unsigned)grid, threads, 0, st>>>(reinterpret_cast<const float*>(src), static_cast<float*>(scratch), cq,
+                                                                    (int)(stride / 4), card, m->nodes[target].lam_off);
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) {
+            bc_set_error("marginal expansion kernel: %s", cudaGetErrorString(e));
+            rc = BC_ECUDA;
+            break;
+        }
+        bc_count_launch();
+        rc = bc_query_batch(m, scratch, cq * card, fmt, nullptr, out + q0 * card, kernel, st);
+    }
+    cudaFreeAsync(scratch, st);
+    return rc;
+}
+
+bool bad_target(const bc_model* m, int target) {
+    if (target < 0 || target >= m->n) {
+        bc_set_error("target node %d outside the model's %d nodes", target, m->n);
+        return true;
+    }
+    return false;
+}
+
+}  // namespace
+
+extern "C" int bc_model_specialize_marginal(bc_model* m, int target, const char* cache_dir) {
+    if (!m || m->device < 0) { bc_set_error("specialize_marginal needs a device model"); return BC_EINVAL; }
+    if (bad_target(m, target)) return BC_EINVAL;
+    return bc_marg_build(m, target, cache_dir);
+}
+
+extern "C" int64_t bc_model_marginal_source(const bc_model* m, int target, char* buf, size_t buf_bytes) {
+    if (!m) { bc_set_error("model is NULL"); return BC_EINVAL; }
+    if (bad_target(m, target)) return BC_EINVAL;
+    if (m->arena.empty()) { bc_set_error("model too large for a specialised kernel"); return BC_ELIMIT; }
+    const std::string s = bc_marginal_generate(*m, target);
+    if (buf && buf_bytes > 0) {
+        const size_t k = s.size() + 1 <= buf_bytes ? s.size() : buf_bytes - 1;
+        std::memcpy(buf, s.data(), k);
+        buf[k] = 0;
+    }
+    return (int64_t)s.size() + 1;
+}
+
+extern "C" uint64_t bc_model_marginal_hash(const bc_model* m, int target) {
+    if (!m || target < 0 || target >= m->n) return 0;
+    return bc_marginal_hash_of(*m, target);
+}
+
+extern "C" int bc_marginal_batch(bc_model* m, const void* desc, size_t nq, int fmt, int target, float* out, int kernel, void* stream) {
+    if (!m || m->device < 0) { bc_set_error("model has no device (host-only model)"); return BC_EINVAL; }
+    if (bad_target(m, target)) return BC_EINVAL;
+    if (fmt != BC_DESC_BITS && fmt != BC_DESC_DENSE_F32) {
+        bc_set_error("bc_marginal_batch reads BITS or DENSE_F32 rows, not format %d", fmt);
+        return BC_EINVAL;
+    }
+    if (nq == 0) return BC_OK;
+    if (!desc || !out) { bc_set_error("desc/out is NULL"); return BC_EINVAL; }
+    BC_CUDA_CHECK(cudaSetDevice(m->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (kernel == BC_KERNEL_SPEC || (kernel == BC_KERNEL_AUTO && bc_marg_attached(m, target)))
+        return bc_marg_launch(m, desc, nq, fmt, target, out, st);
+    return expand_path(m, desc, nq, fmt, target, out, kernel, st);
+}

@@ -27,6 +27,11 @@
 // once (Sethi-Ullman order).  Exact zeros of the CPT (30 % of the shipped DMV / Census entries)
 // emit no instruction; the number of FMAs actually emitted is reported in the header comment of
 // the generated source (BC_SPEC_FFMA) and is what the roofline accounting uses.
+//
+// A second module per (model, target node t) answers GROUP BY t (bc_marginal_generate): out[q][b] for every state b of t.
+// Every subtree off the root -> t path is evaluated upward as above; then a downward chain along the path carries
+//   pi_0 = w_0 * lambda_0 * T_0,   pi_i[c] = w_i[c] * lambda_i[c] * sum_p T_i[c][p] * pi_{i-1}[p],   out = pi_k
+// (lambda_i: product of the messages of a_i's children off the path), again one FMA per non-zero CPT entry.
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
@@ -74,13 +79,15 @@ struct Gen {
     std::vector<std::string> words;  // BITS row words / (dense: unused)
     std::vector<std::string> fmw;    // fan-out mask words
 
-    Gen(const bc_model& mm, bool d) : m(mm), dense(d), kids(mm.n) {
+    const bool use_fan;              // false: fan-out vectors are ignored (the marginal kernels take no fan-out mask)
+
+    Gen(const bc_model& mm, bool d, bool fan = true) : m(mm), dense(d), kids(mm.n), use_fan(fan) {
         std::vector<long long> subtree(m.n, 0);
         for (int v = 1; v < m.n; ++v) kids[m.nodes[v].parent].push_back(v);
         for (int v = m.n - 1; v >= 0; --v) {
             subtree[v] += m.nodes[v].card;
             if (v > 0) subtree[m.nodes[v].parent] += subtree[v];
-            if (m.nodes[v].fan_off >= 0) any_fan = true;
+            if (use_fan && m.nodes[v].fan_off >= 0) any_fan = true;
         }
         for (int v = 0; v < m.n; ++v)
             std::stable_sort(kids[v].begin(), kids[v].end(), [&](int a, int b) { return subtree[a] > subtree[b]; });
@@ -119,7 +126,7 @@ struct Gen {
             else
                 for (int c = 0; c < card; ++c) line("mul.f32 " + lam[c] + ", " + lam[c] + ", " + mk[c] + ";");
         }
-        const bool fan = nd.fan_off >= 0;
+        const bool fan = use_fan && nd.fan_off >= 0;
         std::string pfb;
         if (fan) {
             std::string t = R();
@@ -209,22 +216,79 @@ struct Gen {
         }
         return acc;
     }
+
+    // One step of the downward pass of a marginal along the path root = a_0 -> ... -> a_k = target, at path node v = a_i
+    // (`skip` = a_{i+1}, -1 at the target).  Folds the messages of v's children off the path into lambda, then emits
+    //     pi_i[c] = w_v[c] * lambda[c] * sum_p T_v[c][p] * pi_{i-1}[p]        (root: w_0[c] * lambda[c] * T_0[c])
+    // with one FMA-pipe instruction per non-zero T_v[c][p]; returns pi_i, one register per state of v.
+    std::vector<std::string> path_step(int v, int skip, const std::vector<std::string>& prev) {
+        const BcNodeRec& nd = m.nodes[v];
+        const bool root = v == 0;
+        const int card = nd.card, cols = root ? 1 : nd.card_pa;
+        std::vector<std::string> lam;
+        for (int k : kids[v]) {
+            if (k == skip) continue;
+            std::vector<std::string> mk = message(k);
+            if (lam.empty()) lam = mk;
+            else
+                for (int c = 0; c < card; ++c) line("mul.f32 " + lam[c] + ", " + lam[c] + ", " + mk[c] + ";");
+        }
+        line("// ---- path node " + I(v) + ": card " + I(card) + (root ? " (root)" : ", parent " + I(nd.parent)) +
+             (skip < 0 ? " (target)" : ", next " + I(skip)));
+        const float* T = m.arena.data() + nd.cpt_off;
+        const int stride = root ? 1 : nd.stride;
+        std::vector<std::string> wreg(dense ? ((card + 3) / 4) * 4 : 0);
+        std::string zero;
+        std::vector<std::string> pi(card);
+        for (int c = 0; c < card; ++c) {
+            std::string x;   // lambda[c] * (T_0[c] | sum_p T[c][p] pi[p]): a register, or the immediate T_0[c]
+            if (root) {
+                const float t = T[c];
+                if (t != 0.f) {
+                    ++n_fma;
+                    if (lam.empty()) x = fhex(t);
+                    else { x = F(); line("mul.f32 " + x + ", " + lam[c] + ", " + fhex(t) + ";"); }
+                }
+            } else {
+                for (int p = 0; p < cols; ++p) {
+                    const float t = T[(size_t)c * stride + p];
+                    if (t == 0.f) continue;
+                    ++n_fma;
+                    if (x.empty()) { x = F(); line("mul.f32 " + x + ", " + prev[p] + ", " + fhex(t) + ";"); }
+                    else line("fma.rn.f32 " + x + ", " + prev[p] + ", " + fhex(t) + ", " + x + ";");
+                }
+                if (!x.empty() && !lam.empty()) line("mul.f32 " + x + ", " + x + ", " + lam[c] + ";");
+            }
+            if (x.empty()) {   // an all-zero CPT row: the state holds no mass
+                if (zero.empty()) { zero = F(); line("mov.f32 " + zero + ", 0f00000000;"); }
+                pi[c] = zero;
+                continue;
+            }
+            pi[c] = F();
+            if (dense) {
+                const int j = c / 4;
+                if (wreg[4 * j].empty()) {
+                    std::string a = F(), b = F(), c2 = F(), d = F();
+                    line("ld.global.nc.v4.f32 {" + a + ", " + b + ", " + c2 + ", " + d + "}, [%rrow+" + I(4LL * (nd.lam_off + 4 * j)) + "];");
+                    wreg[4 * j] = a; wreg[4 * j + 1] = b; wreg[4 * j + 2] = c2; wreg[4 * j + 3] = d;
+                }
+                line("mul.f32 " + pi[c] + ", " + wreg[c] + ", " + x + ";");
+            } else {
+                line("selp.f32 " + pi[c] + ", " + x + ", 0f00000000, " + bit_pred(v, c) + ";");
+            }
+        }
+        return pi;
+    }
 };
 
-std::string gen_kernel(const bc_model& m, bool dense, int threads, int min_blocks, long long* n_fma) {
-    Gen g(m, dense);
-    const int sync_every = env_int("BC_SPEC_SYNC_EVERY", 0);
-    g.sync_every = sync_every;
+// Wraps the straight-line body of `g` in the query loop of one entry point and stores `res`, res.size() consecutive floats
+// per query (row q at out + 4 * res.size() * q).
+std::string gen_entry(const bc_model& m, Gen& g, const char* name, bool dense, int threads, int min_blocks,
+                      const std::vector<std::string>& res) {
+    const int sync_every = g.sync_every;
     const int words = m.bits_words;
-    if (!dense)
-        for (int w = 0; w < words; ++w) g.words.push_back(g.R());
-    for (int w = 0; w < m.mask_words; ++w) g.fmw.push_back(g.R());
-    const std::string res = g.message(0)[0];
-    if (n_fma) *n_fma = g.n_fma;
-
     const bool dynamic = env_int("BC_SPEC_DYNAMIC", 1) != 0;
     std::string s;
-    const char* name = dense ? "bc_spec_dense" : "bc_spec_bits";
     s += std::string(".visible .entry ") + name +
          "(\n    .param .u64 p_desc,\n    .param .u64 p_stride,\n    .param .u64 p_fmask,\n    .param .u64 p_out,\n"
          "    .param .u64 p_nq,\n    .param .u64 p_ctr\n)\n.maxntid " + I(threads) + ", 1, 1\n.minnctapersm " + I(min_blocks) + "\n{\n";
@@ -319,9 +383,11 @@ std::string gen_kernel(const bc_model& m, bool dense, int threads, int min_block
         }
     }
     s += g.out;
-    e("shl.b64 %rtmp, %rq, 2;");
+    if (res.size() == 1) e("shl.b64 %rtmp, %rq, 2;");
+    else e("mul.lo.u64 %rtmp, %rq, " + I(4LL * (long long)res.size()) + ";");
     e("add.u64 %rtmp, %rtmp, %rout;");
-    e(std::string(clamp ? "@%pvalid " : "") + "st.global.f32 [%rtmp], " + res + ";");
+    for (size_t b = 0; b < res.size(); ++b)
+        e(std::string(clamp ? "@%pvalid " : "") + "st.global.f32 [%rtmp" + (b ? "+" + I(4LL * (long long)b) : "") + "], " + res[b] + ";");
     if (!dynamic) {
         e("add.u64 %rq, %rq, %rstep;");
         if (sync_every > 0) e("add.u64 %rqb, %rqb, %rstep;");
@@ -346,6 +412,34 @@ std::string gen_kernel(const bc_model& m, bool dense, int threads, int min_block
     }
     s += "DONE:\n    ret;\n}\n\n";
     return s;
+}
+
+std::string gen_kernel(const bc_model& m, bool dense, int threads, int min_blocks, long long* n_fma) {
+    Gen g(m, dense);
+    g.sync_every = env_int("BC_SPEC_SYNC_EVERY", 0);
+    if (!dense)
+        for (int w = 0; w < m.bits_words; ++w) g.words.push_back(g.R());
+    for (int w = 0; w < m.mask_words; ++w) g.fmw.push_back(g.R());
+    const std::string res = g.message(0)[0];
+    if (n_fma) *n_fma = g.n_fma;
+    return gen_entry(m, g, dense ? "bc_spec_dense" : "bc_spec_bits", dense, threads, min_blocks, {res});
+}
+
+// The marginal of `target`: the upward pass of every subtree off the root -> target path (Gen::message), then the downward
+// chain of path_step, then card(target) stores per query.
+std::string gen_marginal_kernel(const bc_model& m, int target, bool dense, int threads, int min_blocks, long long* n_fma) {
+    Gen g(m, dense, false);
+    g.sync_every = env_int("BC_SPEC_SYNC_EVERY", 0);
+    if (!dense)
+        for (int w = 0; w < m.bits_words; ++w) g.words.push_back(g.R());
+    std::vector<int> path;
+    for (int v = target; v > 0; v = m.nodes[v].parent) path.push_back(v);
+    path.push_back(0);
+    std::reverse(path.begin(), path.end());
+    std::vector<std::string> pi;
+    for (size_t i = 0; i < path.size(); ++i) pi = g.path_step(path[i], i + 1 < path.size() ? path[i + 1] : -1, pi);
+    if (n_fma) *n_fma = g.n_fma;
+    return gen_entry(m, g, dense ? "bc_marg_dense" : "bc_marg_bits", dense, threads, min_blocks, pi);
 }
 
 }  // namespace
@@ -398,5 +492,41 @@ uint64_t bc_spec_hash_of(const bc_model& m) {
     for (const BcNodeRec& r : m.nodes) mix(&r, sizeof(r));
     mix(m.arena.data(), m.arena.size() * sizeof(float));
     mix(m.fan.data(), m.fan.size() * sizeof(float));
+    return h;
+}
+
+// Module of the marginal kernels of one target: bc_marg_bits / bc_marg_dense, the same loop, geometry and work counter as the
+// bc_spec_* entries, out[q][b] for b < card(target).  The header's BC_SPEC_FFMA counts the FMA-pipe instructions that carry a
+// CPT entry: one per non-zero entry of the whole tree, as in the spec module.
+std::string bc_marginal_generate(const bc_model& m, int target) {
+    int threads, min_blocks;
+    bc_spec_geometry(m, &threads, &min_blocks);
+    long long f1 = 0, f2 = 0;
+    std::string k1 = gen_marginal_kernel(m, target, false, threads, min_blocks, &f1);
+    std::string k2 = gen_marginal_kernel(m, target, true, threads, min_blocks, &f2);
+    std::string path;
+    for (int v = target; v >= 0; v = m.nodes[v].parent) path = I(v) + (path.empty() ? "" : " -> " + path);
+    std::string s;
+    s += "//\n// Generated by bayescard_b200 spec_codegen, marginal generator (version " + I(BC_MARGINAL_VERSION) + ", codegen version " +
+         I(BC_CODEGEN_VERSION) + ") -- do not edit.\n";
+    s += "// nodes: " + I(m.n) + "  target: " + I(target) + "  card: " + I(m.nodes[target].card) + "  path: " + path + "\n";
+    s += "// BC_SPEC_THREADS=" + I(threads) + " BC_SPEC_MIN_BLOCKS=" + I(min_blocks) + " BC_SPEC_FFMA=" + I(f1) + "\n//\n";
+    s += ".version 8.7\n.target sm_100a\n.address_size 64\n\n";
+    // {threads per CTA, results per query (= card of the target), marginal generator version, target}
+    s += ".visible .global .align 4 .u32 bc_marg_meta[4] = {" + I(threads) + ", " + I(m.nodes[target].card) + ", " +
+         I(BC_MARGINAL_VERSION) + ", " + I(target) + "};\n\n";
+    s += k1;
+    s += k2;
+    return s;
+}
+
+uint64_t bc_marginal_hash_of(const bc_model& m, int target) {
+    uint64_t h = bc_spec_hash_of(m);
+    auto mix = [&](const void* p, size_t n) {
+        const unsigned char* b = static_cast<const unsigned char*>(p);
+        for (size_t i = 0; i < n; ++i) { h ^= b[i]; h *= 1099511628211ull; }
+    };
+    const int tag[2] = {BC_MARGINAL_VERSION, target};
+    mix(tag, sizeof(tag));
     return h;
 }

@@ -242,6 +242,34 @@ class PredicateCompiler:
                     bins_out[attr], wts_out[attr] = [int(p[0])], np.asarray([p[1]], dtype=np.float64)
         return bins_out, wts_out
 
+    def select_values(self, attr: str, val) -> Optional[np.ndarray]:
+        """Which original values of categorical column ``attr`` a predicate value selects, by ``decode``'s rules: a bool
+        mask over the encoding's keys in encoding order, or ``None`` where ``decode`` finds the predicate undecodable.
+        A scalar selects itself; a list its known members (unknown ones are dropped); a ``(lo, hi)`` tuple every value
+        inside the range except the column's null value."""
+        col = self.cols[attr]
+        if col.enc is None:
+            return None
+        keys = list(col.pair)
+        if type(val) == tuple:
+            lo, hi = val[0], val[1]
+            if col.num_vals is not None and isinstance(lo, (int, float)) and isinstance(hi, (int, float)):
+                keep = (col.num_vals >= lo) & (col.num_vals <= hi)
+                if col.has_null:
+                    keep &= col.num_vals != col.null
+            else:
+                keep = np.asarray([not (col.has_null and k == col.null) and lo <= k <= hi for k in keys], dtype=bool)
+            return keep if keep.any() else None
+        if type(val) == list:
+            if len(val) == 0:
+                return None
+            chosen = set(v for v in val if v in col.pair)
+        else:
+            if val not in col.pair:
+                return None
+            chosen = {val}
+        return np.asarray([k in chosen for k in keys], dtype=bool)
+
     # ------------------------------------------------------------------ stage 2
     @staticmethod
     def _unit_bins(b: Sequence[int], w) -> bool:

@@ -10,7 +10,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import threading
-from typing import List, Optional, Sequence
+from typing import Dict, List, Optional, Sequence
 
 import numpy as np
 
@@ -45,6 +45,8 @@ class DeviceModel:
         self.flops_dense = int(lib.bc_model_flops_dense(h))
         self.max_card = int(card.max())
         self.spec_error: Optional[str] = None
+        self.marginal_error: Dict[int, str] = {}   # target node -> why its specialised marginal kernel is missing
+        self._marginal_built: Dict[int, bool] = {}
         if specialize and device >= 0:
             try:
                 self.specialize(cache_dir)
@@ -105,6 +107,68 @@ class DeviceModel:
             image = image + b"\0"  # PTX must be NUL terminated
         buf = C.create_string_buffer(image, len(image))
         L.check(L.lib().bc_model_load_cubin(self._h, buf, len(image)))
+
+    # ------------------------------------------------------------------ GROUP BY one column (per-state marginals)
+    def _check_node(self, node: int) -> int:
+        node = int(node)
+        if not 0 <= node < self.n_nodes:
+            raise ValueError(f"node {node} outside the model's {self.n_nodes} nodes")
+        return node
+
+    def specialize_marginal(self, node: int, cache_dir: Optional[str] = None) -> bool:
+        """Attach the specialised marginal kernel of ``node`` (built on the first call, then kept).  A failure is
+        recorded in ``marginal_error[node]`` and not retried; ``marginal_batch`` then serves the node by expansion."""
+        node = self._check_node(node)
+        if node not in self._marginal_built:
+            cache_dir = L.SPEC_CACHE_DIR if cache_dir is None else cache_dir
+            try:
+                L.check(L.lib().bc_model_specialize_marginal(self._h, node, cache_dir.encode() if cache_dir else None))
+                self._marginal_built[node] = True
+            except L.BayesCardError as e:
+                self.marginal_error[node] = str(e)
+                self._marginal_built[node] = False
+        return self._marginal_built[node]
+
+    def marginal_source(self, node: int) -> str:
+        lib = L.lib()
+        node = self._check_node(node)
+        n = lib.bc_model_marginal_source(self._h, node, None, 0)
+        if n < 0:
+            L.check(int(n))
+        buf = C.create_string_buffer(int(n))
+        lib.bc_model_marginal_source(self._h, node, buf, int(n))
+        return buf.value.decode()
+
+    def marginal_hash(self, node: int) -> int:
+        return int(L.lib().bc_model_marginal_hash(self._h, self._check_node(node)))
+
+    def run_marginal_device(self, desc_ptr: int, n: int, fmt: int, node: int, out_ptr: int, kernel: int = L.KERNEL_AUTO,
+                            stream: int = 0) -> None:
+        """``bc_marginal_batch`` on DEVICE buffers: ``out`` receives ``[n][card(node)]`` fp32."""
+        L.check(L.lib().bc_marginal_batch(self._h, desc_ptr or None, n, fmt, int(node), out_ptr or None, kernel, stream or None))
+
+    def run_marginal_host(self, desc: np.ndarray, fmt: int, node: int, kernel: int = L.KERNEL_AUTO) -> np.ndarray:
+        """BITS / DENSE_F32 rows from the host -> ``ndarray [n, card(node)]`` fp32: the per-state mass of ``node`` under
+        each row.  torch moves the buffers; the work is ``bc_marginal_batch``."""
+        node = self._check_node(node)
+        stride = self.desc_stride(fmt)
+        desc = np.ascontiguousarray(desc)
+        n = desc.nbytes // stride
+        if desc.nbytes != n * stride:
+            raise ValueError(f"descriptor buffer of {desc.nbytes} B is not a multiple of the row stride {stride}")
+        card = int(self.tm.card[node])
+        if n == 0 or self.device < 0:   # (the library still validates the arguments)
+            L.check(L.lib().bc_marginal_batch(self._h, None, n, fmt, node, None, kernel, None))
+            return np.zeros((n, card), dtype=np.float32)
+        import torch
+
+        dev = torch.device("cuda", self.device)
+        with torch.cuda.device(dev):
+            d_desc = torch.from_numpy(desc.reshape(-1).view(np.uint8)).to(dev)
+            d_out = torch.empty(n * card, dtype=torch.float32, device=dev)
+            self.run_marginal_device(d_desc.data_ptr(), n, fmt, node, d_out.data_ptr(), kernel,
+                                     torch.cuda.current_stream().cuda_stream)
+            return d_out.cpu().numpy().reshape(n, card)
 
     # ------------------------------------------------------------------ geometry
     def desc_stride(self, fmt: int) -> int:

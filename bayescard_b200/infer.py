@@ -31,6 +31,7 @@ class VariableEliminationB200:
             self.dev = DeviceModel(tm, int(device), specialize=specialize)
             self._single = self.dev
         self.kernel = kernel
+        self.specialize = specialize
         self.root = tm.infer_names[0]
         self.fanouts = tm.fanouts
 
@@ -66,6 +67,25 @@ class VariableEliminationB200:
         for i, (q, f) in enumerate(zip(queries, fanout_attrs)):
             if not any(k in self.tm._index for k in list(q) + list(f)):
                 out[i] = 0.0
+        return out
+
+    def marginal_batch(self, decoded, name: str, kernel: Optional[int] = None) -> np.ndarray:
+        """GROUP BY ``name``: ``[len(decoded), card]`` fp64, row i = the per-state mass of column ``name`` under the
+        already decoded query i (``bc_marginal_batch``; its row sums are what ``run_decoded`` returns).  The first call for
+        a column attaches its specialised marginal kernel; a sharded machine answers on its first replica."""
+        v = self.tm._index[name]
+        kernel = self.kernel if kernel is None else kernel
+        dm = self._single
+        if self.specialize and kernel in (L.KERNEL_AUTO, L.KERNEL_SPEC) and dm.device >= 0:
+            dm.specialize_marginal(v)
+        out = np.zeros((len(decoded), int(self.tm.card[v])), dtype=np.float64)
+        if len(decoded) == 0:
+            return out
+        b_idx, b_desc, d_idx, d_desc, _ = self.compiler.pack(decoded)
+        if len(b_idx):
+            out[b_idx] = dm.run_marginal_host(b_desc, L.DESC_BITS, v, kernel)
+        if len(d_idx):
+            out[d_idx] = dm.run_marginal_host(d_desc, L.DESC_DENSE_F32, v, kernel)
         return out
 
     @staticmethod

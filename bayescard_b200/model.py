@@ -169,6 +169,78 @@ class Bayescard_BN:
             out[dense_idx] = m.dev.run_host(dense_rows, L.DESC_DENSE_F32, None, m.kernel)
         return out if return_prob else out * self.nrows
 
+    # ------------------------------------------------------------------ GROUP BY one column
+    def groupby_batch(self, queries: Sequence[dict], column: str, return_prob: bool = False):
+        """``SELECT column, COUNT(*) ... WHERE P GROUP BY column`` for a batch of predicate dicts ``P``: returns ``(keys,
+        est)`` with ``est[i, j]`` the estimate of group ``keys[j]`` under query i -- one pass per query on the GPU
+        (``bc_marginal_batch``) instead of one query per group value.
+
+        * A categorical column with an encoding: the keys are its original values in encoding order and
+          ``est(v) = nrows * M[bin(v)] * weight(v)``, which is ``self.query({**P_without_column, column: v})``.  M is the
+          per-bin mass without the predicate on ``column``; values that predicate does not select get 0.
+        * A continuous column, or one without an encoding: the keys are the bins (continuous: the bin's interval from
+          ``mapping``); the predicate on ``column`` stays, with its coverage weights, and ``est(b) = nrows * M[b]``.
+
+        Undecodable queries give a zero row; a query without predicates gives the column's marginal."""
+        m = self._machine()
+        v = self.tree._index.get(column)
+        if v is None:
+            raise ValueError(f"column {column!r} is not a node of this model")
+        col = m.compiler.cols[column]
+        categorical = col.kind != "continuous" and col.enc is not None
+        if categorical:
+            keys = list(col.pair)
+            key_bin = np.asarray([col.pair[k][0] for k in keys], dtype=np.int64)
+            key_wt = np.asarray([col.pair[k][1] for k in keys], dtype=np.float64)
+        elif col.kind == "continuous" and col.edges is not None:
+            keys = [tuple(col.edges[b]) for b in range(int(self.tree.card[v]))]
+        else:
+            keys = list(range(int(self.tree.card[v])))
+        est = np.zeros((len(queries), len(keys)), dtype=np.float64)
+        decoded, keep, sel = [], [], []
+        for i, q in enumerate(queries):
+            if categorical:
+                s = np.ones(len(keys), dtype=bool)
+                if column in q:
+                    s = m.compiler.select_values(column, q[column])
+                    if s is None:
+                        continue
+                q = {k: x for k, x in q.items() if k != column}
+                sel.append(s)
+            b, w = m.compiler.decode(q)
+            if b is None:
+                if categorical:
+                    sel.pop()
+                continue
+            decoded.append((b, w))
+            keep.append(i)
+        if decoded:
+            M = m.marginal_batch(decoded, column)
+            if categorical:
+                est[keep] = M[:, key_bin] * key_wt[None, :] * np.asarray(sel)
+            else:
+                est[keep] = M
+        return keys, (est if return_prob else est * self.nrows)
+
+    def groupby(self, query: dict, column: str, return_prob: bool = False) -> Dict[Any, float]:
+        """One query of :meth:`groupby_batch`: ``{key: estimate}``."""
+        keys, est = self.groupby_batch([query], column, return_prob)
+        return {k: float(e) for k, e in zip(keys, est[0])}
+
+    def groupby_sql_batch(self, sqls: Sequence[str], return_prob: bool = False) -> List[Dict[Any, float]]:
+        """``SELECT a, COUNT(*) FROM t [WHERE ...] GROUP BY a`` texts -> one ``{key: estimate}`` per text; the texts that
+        group by the same column are answered in one batch."""
+        from .sql_front import parse_groupby_single_table
+
+        parsed = [parse_groupby_single_table(s, self) for s in sqls]
+        out: List[Dict[Any, float]] = [{} for _ in sqls]
+        for column in dict.fromkeys(c for _, c in parsed):
+            idx = [i for i, (_, c) in enumerate(parsed) if c == column]
+            keys, est = self.groupby_batch([parsed[i][0] for i in idx], column, return_prob)
+            for j, i in enumerate(idx):
+                out[i] = {k: float(e) for k, e in zip(keys, est[j])}
+        return out
+
     def close(self):
         if getattr(self, "_sqlc", None) is not None:
             self._sqlc.close()

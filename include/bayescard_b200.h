@@ -164,6 +164,29 @@ BC_API int bc_query_batch(bc_model* m, const void* desc, size_t n_queries, int d
 BC_API int bc_query_batch_host(bc_model* m, const void* desc, size_t n_queries, int desc_format,
                         const uint32_t* fanout_mask, float* out_prob, int kernel);
 
+/* ---- GROUP BY one column: per-state counts of a target node under each query's predicates ---------------------------
+ * Replaces the per-value loop `[bn.query({**P, a: v}) for v in values]` over Bayescard_BN.query (Models/Bayescard_BN.py:496)
+ * with ONE pass per query: for the target node t (topological index) and each row's weights w_v,
+ *     out[q][b] = sum_{x : x_t = b} prod_v w_v[x_v] T_v[x_v, x_pa(v)]          b = 0 .. card(t) - 1
+ * so w_t restricts the groups and sum_b out[q][b] is the out_prob[q] of bc_query_batch on the same row.  out is contiguous
+ * fp32 [n_queries][card(t)].  Rows are BITS or DENSE_F32; there is no fan-out mask (fan-out columns are unconstrained).
+ * DEVICE pointers, stream ordered.  kernel:
+ *   BC_KERNEL_AUTO   the specialised marginal kernel of t when it is attached, otherwise the expansion below
+ *   BC_KERNEL_SPEC   the specialised marginal kernel of t; BC_ECOMPILE when it is not attached
+ *   any other id     the expansion through that kernel: every row becomes card(t) rows (the target's weights restricted
+ *                    to one state each, built on the device in chunks of <= 256 MB), evaluated q-major by bc_query_batch
+ * BC_EINVAL for a target outside [0, n_nodes), a RANGE_* or unknown format, or a host-only model; n_queries == 0 is BC_OK
+ * with no launch.  Results below the fp32 range are not carried (no scaled form). */
+BC_API int bc_marginal_batch(bc_model* m, const void* desc, size_t n_queries, int desc_format, int target, float* out,
+                             int kernel, void* stream);
+/* Build (or load "<cache_dir>/marg_<hash>.cubin") the specialised marginal kernel of one target node: straight-line sm_100a
+ * code like bc_model_specialize's, attached through the driver JIT; one module per target, kept on the model. */
+BC_API int bc_model_specialize_marginal(bc_model* m, int target, const char* cache_dir);
+/* Its generated PTX (host-only models too; returns the bytes needed including the NUL) and the hash that names its cache
+ * entry (model, target and marginal generator version; 0 for a target out of range). */
+BC_API int64_t bc_model_marginal_source(const bc_model* m, int target, char* buf, size_t buf_bytes);
+BC_API uint64_t bc_model_marginal_hash(const bc_model* m, int target);
+
 /* Device-side descriptor conversion (stream ordered, DEVICE pointers): RANGE_U8 / RANGE_U16 -> BITS. */
 BC_API int bc_convert_desc(bc_model* m, const void* src, int src_format, void* dst, int dst_format, size_t n_queries,
                     void* stream);
