@@ -16,7 +16,8 @@
 #define BC_VERSION_STRING "bayescard_b200 0.1.0 (sm_100a)"
 #define BC_CODEGEN_VERSION 10
 #define BC_SPEC_CTR_SLOTS 256
-#define BC_MARGINAL_VERSION 1   // marginal kernels (bc_marg_*): part of their cache name, independent of BC_CODEGEN_VERSION
+#define BC_MARGINAL_VERSION 2   // marginal kernels (bc_marg_*): part of their cache name, independent of BC_CODEGEN_VERSION;
+                                // 2: the kernels apply the fan-out mask
 
 // One record per node, copied to the device and (by K1) into shared memory.  32 bytes.
 struct BcNodeRec {
@@ -161,5 +162,6 @@ std::string bc_marginal_generate(const bc_model& m, int target);
 uint64_t bc_marginal_hash_of(const bc_model& m, int target);
 int bc_marg_build(bc_model* m, int target, const char* cache_dir);
 bool bc_marg_attached(bc_model* m, int target);
-int bc_marg_launch(bc_model* m, const void* desc, size_t nq, int fmt, int target, float* out, cudaStream_t stream);
+int bc_marg_launch(bc_model* m, const void* desc, size_t nq, int fmt, const uint32_t* fan_mask, int target, float* out,
+                   cudaStream_t stream);
 void bc_marg_free(bc_model* m);

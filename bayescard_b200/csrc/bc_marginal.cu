@@ -1,10 +1,12 @@
-// GROUP BY on one column: out[q][b] = sum_{x : x_t = b} prod_v w_v[x_v] T_v[x_v, x_pa(v)] for every state b of a target node t.
+// GROUP BY on one column: out[q][b] = sum_{x : x_t = b} prod_v w_v[x_v] T_v[x_v, x_pa(v)] for every state b of a target node t,
+// with w_v multiplied by fanouts[v] where bit v of query q's fan-out mask is set (bc_expectation_marginal_batch).
 //
 // Two paths (see include/bayescard_b200.h, bc_marginal_batch):
 //   - the specialised marginal kernel of (model, t) (spec_codegen.cc / spec_jit.cu): one upward pass plus one downward
 //     chain along the root -> t path per query, card(t) results per thread;
 //   - the expansion, for every model the existing kernels serve: each row becomes card(t) rows, row b with the target's
-//     weights restricted to state b, evaluated q-major by bc_query_batch, so its results already are out[q][b].
+//     weights restricted to state b (and the query's mask row), evaluated q-major by bc_query_batch, so its results already
+//     are out[q][b].
 #include <cstring>
 
 #include "bc_internal.h"
@@ -47,39 +49,58 @@ __global__ void expand_dense_kernel(const float* __restrict__ src, float* __rest
     }
 }
 
-constexpr size_t kExpandBytes = 256u << 20;   // bound on the expanded rows of one chunk
+// Fan-out mask: row (q, b) = mask row q, for each of the card rows of query q.
+__global__ void expand_mask_kernel(const uint32_t* __restrict__ src, uint32_t* __restrict__ dst, size_t nq, int words, int card) {
+    const size_t total = nq * (size_t)card * words;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x)
+        dst[i] = src[(i / ((size_t)card * words)) * words + i % words];
+}
 
-int expand_path(bc_model* m, const void* desc, size_t nq, int fmt, int target, float* out, int kernel, cudaStream_t st) {
+constexpr size_t kExpandBytes = 256u << 20;   // bound on the expanded rows (and mask rows) of one chunk
+
+int expand_path(bc_model* m, const void* desc, size_t nq, int fmt, const uint32_t* fan_mask, int target, float* out, int kernel,
+                cudaStream_t st) {
     const int card = m->nodes[target].card;
     const size_t stride = (size_t)bc_model_desc_stride(m, fmt);
-    const size_t row_bytes = stride * card;   // expanded bytes per query
+    const size_t mask_stride = fan_mask ? 4 * (size_t)m->mask_words : 0;
+    const size_t row_bytes = (stride + mask_stride) * card;   // expanded bytes per query
     size_t chunk = kExpandBytes / row_bytes;
     if (chunk < 1) chunk = 1;
     if (chunk > nq) chunk = nq;
     void* scratch = nullptr;
     BC_CUDA_CHECK(cudaMallocAsync(&scratch, chunk * row_bytes, st));
+    // the expanded mask rows follow the descriptor rows (stride is a multiple of 16 bytes)
+    uint32_t* mask_scratch = fan_mask ? reinterpret_cast<uint32_t*>(static_cast<unsigned char*>(scratch) + chunk * stride * card) : nullptr;
     const int threads = 256;
+    auto grid_of = [&](size_t elems) {
+        long long grid = (long long)((elems + threads - 1) / threads);
+        return (unsigned)(grid > (long long)m->sm_count * 16 ? (long long)m->sm_count * 16 : grid);
+    };
     int rc = BC_OK;
     for (size_t q0 = 0; q0 < nq && rc == BC_OK; q0 += chunk) {
         const size_t cq = nq - q0 < chunk ? nq - q0 : chunk;
-        const size_t elems = cq * row_bytes / 4;
-        long long grid = (long long)((elems + threads - 1) / threads);
-        if (grid > (long long)m->sm_count * 16) grid = (long long)m->sm_count * 16;
+        const unsigned grid = grid_of(cq * card * stride / 4);
         const unsigned char* src = static_cast<const unsigned char*>(desc) + q0 * stride;
         if (fmt == BC_DESC_BITS)
-            expand_bits_kernel<<<(unsigned)grid, threads, 0, st>>>(reinterpret_cast<const uint32_t*>(src), static_cast<uint32_t*>(scratch),
-                                                                   cq, (int)(stride / 4), card, m->bits[target].bit_off);
+            expand_bits_kernel<<<grid, threads, 0, st>>>(reinterpret_cast<const uint32_t*>(src), static_cast<uint32_t*>(scratch), cq,
+                                                         (int)(stride / 4), card, m->bits[target].bit_off);
         else
-            expand_dense_kernel<<<(unsigned)grid, threads, 0, st>>>(reinterpret_cast<const float*>(src), static_cast<float*>(scratch), cq,
-                                                                    (int)(stride / 4), card, m->nodes[target].lam_off);
+            expand_dense_kernel<<<grid, threads, 0, st>>>(reinterpret_cast<const float*>(src), static_cast<float*>(scratch), cq,
+                                                          (int)(stride / 4), card, m->nodes[target].lam_off);
         cudaError_t e = cudaGetLastError();
+        if (e == cudaSuccess && fan_mask) {
+            bc_count_launch();
+            expand_mask_kernel<<<grid_of(cq * card * m->mask_words), threads, 0, st>>>(fan_mask + q0 * m->mask_words, mask_scratch, cq,
+                                                                                       m->mask_words, card);
+            e = cudaGetLastError();
+        }
         if (e != cudaSuccess) {
             bc_set_error("marginal expansion kernel: %s", cudaGetErrorString(e));
             rc = BC_ECUDA;
             break;
         }
         bc_count_launch();
-        rc = bc_query_batch(m, scratch, cq * card, fmt, nullptr, out + q0 * card, kernel, st);
+        rc = bc_query_batch(m, scratch, cq * card, fmt, mask_scratch, out + q0 * card, kernel, st);
     }
     cudaFreeAsync(scratch, st);
     return rc;
@@ -119,7 +140,8 @@ extern "C" uint64_t bc_model_marginal_hash(const bc_model* m, int target) {
     return bc_marginal_hash_of(*m, target);
 }
 
-extern "C" int bc_marginal_batch(bc_model* m, const void* desc, size_t nq, int fmt, int target, float* out, int kernel, void* stream) {
+extern "C" int bc_expectation_marginal_batch(bc_model* m, const void* desc, size_t nq, int fmt, const uint32_t* fanout_mask, int target,
+                                             float* out, int kernel, void* stream) {
     if (!m || m->device < 0) { bc_set_error("model has no device (host-only model)"); return BC_EINVAL; }
     if (bad_target(m, target)) return BC_EINVAL;
     if (fmt != BC_DESC_BITS && fmt != BC_DESC_DENSE_F32) {
@@ -131,6 +153,10 @@ extern "C" int bc_marginal_batch(bc_model* m, const void* desc, size_t nq, int f
     BC_CUDA_CHECK(cudaSetDevice(m->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (kernel == BC_KERNEL_SPEC || (kernel == BC_KERNEL_AUTO && bc_marg_attached(m, target)))
-        return bc_marg_launch(m, desc, nq, fmt, target, out, st);
-    return expand_path(m, desc, nq, fmt, target, out, kernel, st);
+        return bc_marg_launch(m, desc, nq, fmt, fanout_mask, target, out, st);
+    return expand_path(m, desc, nq, fmt, fanout_mask, target, out, kernel, st);
+}
+
+extern "C" int bc_marginal_batch(bc_model* m, const void* desc, size_t nq, int fmt, int target, float* out, int kernel, void* stream) {
+    return bc_expectation_marginal_batch(m, desc, nq, fmt, nullptr, target, out, kernel, stream);
 }

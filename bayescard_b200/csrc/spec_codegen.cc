@@ -31,7 +31,8 @@
 // A second module per (model, target node t) answers GROUP BY t (bc_marginal_generate): out[q][b] for every state b of t.
 // Every subtree off the root -> t path is evaluated upward as above; then a downward chain along the path carries
 //   pi_0 = w_0 * lambda_0 * T_0,   pi_i[c] = w_i[c] * lambda_i[c] * sum_p T_i[c][p] * pi_{i-1}[p],   out = pi_k
-// (lambda_i: product of the messages of a_i's children off the path), again one FMA per non-zero CPT entry.
+// (lambda_i: product of the messages of a_i's children off the path), again one FMA per non-zero CPT entry.  Both passes
+// apply the fan-out mask (p_fmask) as the spec module does: bit v multiplies w_v by fanouts[v].
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
@@ -79,15 +80,13 @@ struct Gen {
     std::vector<std::string> words;  // BITS row words / (dense: unused)
     std::vector<std::string> fmw;    // fan-out mask words
 
-    const bool use_fan;              // false: fan-out vectors are ignored (the marginal kernels take no fan-out mask)
-
-    Gen(const bc_model& mm, bool d, bool fan = true) : m(mm), dense(d), kids(mm.n), use_fan(fan) {
+    Gen(const bc_model& mm, bool d) : m(mm), dense(d), kids(mm.n) {
         std::vector<long long> subtree(m.n, 0);
         for (int v = 1; v < m.n; ++v) kids[m.nodes[v].parent].push_back(v);
         for (int v = m.n - 1; v >= 0; --v) {
             subtree[v] += m.nodes[v].card;
             if (v > 0) subtree[m.nodes[v].parent] += subtree[v];
-            if (use_fan && m.nodes[v].fan_off >= 0) any_fan = true;
+            if (m.nodes[v].fan_off >= 0) any_fan = true;
         }
         for (int v = 0; v < m.n; ++v)
             std::stable_sort(kids[v].begin(), kids[v].end(), [&](int a, int b) { return subtree[a] > subtree[b]; });
@@ -103,6 +102,14 @@ struct Gen {
             out += "    bar.sync 0;\n";
             since_sync = 0;
         }
+    }
+
+    // The predicate "bit v of the query's fan-out mask is set" (a NULL mask loads words of 0: never set).
+    std::string fan_pred(int v) {
+        std::string t = R(), p = P();
+        line("and.b32 " + t + ", " + fmw[v >> 5] + ", " + I(1LL << (v & 31)) + ";");
+        line("setp.ne.u32 " + p + ", " + t + ", 0;");
+        return p;
     }
 
     std::string bit_pred(int v, int c) {
@@ -126,14 +133,8 @@ struct Gen {
             else
                 for (int c = 0; c < card; ++c) line("mul.f32 " + lam[c] + ", " + lam[c] + ", " + mk[c] + ";");
         }
-        const bool fan = use_fan && nd.fan_off >= 0;
-        std::string pfb;
-        if (fan) {
-            std::string t = R();
-            pfb = P();
-            line("and.b32 " + t + ", " + fmw[v >> 5] + ", " + I(1LL << (v & 31)) + ";");
-            line("setp.ne.u32 " + pfb + ", " + t + ", 0;");
-        }
+        const bool fan = nd.fan_off >= 0;
+        const std::string pfb = fan ? fan_pred(v) : std::string();
         const float* T = m.arena.data() + nd.cpt_off;
         const int stride = root ? 1 : nd.stride;
         auto Tat = [&](int c, int p) { return root ? T[c] : T[(size_t)c * stride + p]; };
@@ -220,7 +221,9 @@ struct Gen {
     // One step of the downward pass of a marginal along the path root = a_0 -> ... -> a_k = target, at path node v = a_i
     // (`skip` = a_{i+1}, -1 at the target).  Folds the messages of v's children off the path into lambda, then emits
     //     pi_i[c] = w_v[c] * lambda[c] * sum_p T_v[c][p] * pi_{i-1}[p]        (root: w_0[c] * lambda[c] * T_0[c])
-    // with one FMA-pipe instruction per non-zero T_v[c][p]; returns pi_i, one register per state of v.
+    // with one FMA-pipe instruction per non-zero T_v[c][p]; returns pi_i, one register per state of v.  A path node with a
+    // fan-out vector multiplies each state by fanouts[v][c] under its mask bit (@p mul, or a selp between two immediates at a
+    // root without lambda), so a query without that bit computes exactly what the kernel without fan-out does.
     std::vector<std::string> path_step(int v, int skip, const std::vector<std::string>& prev) {
         const BcNodeRec& nd = m.nodes[v];
         const bool root = v == 0;
@@ -235,6 +238,8 @@ struct Gen {
         }
         line("// ---- path node " + I(v) + ": card " + I(card) + (root ? " (root)" : ", parent " + I(nd.parent)) +
              (skip < 0 ? " (target)" : ", next " + I(skip)));
+        const bool fan = nd.fan_off >= 0;
+        const std::string pfb = fan ? fan_pred(v) : std::string();
         const float* T = m.arena.data() + nd.cpt_off;
         const int stride = root ? 1 : nd.stride;
         std::vector<std::string> wreg(dense ? ((card + 3) / 4) * 4 : 0);
@@ -246,8 +251,14 @@ struct Gen {
                 const float t = T[c];
                 if (t != 0.f) {
                     ++n_fma;
-                    if (lam.empty()) x = fhex(t);
-                    else { x = F(); line("mul.f32 " + x + ", " + lam[c] + ", " + fhex(t) + ";"); }
+                    if (lam.empty() && !fan) x = fhex(t);
+                    else if (lam.empty()) {   // fp32 T_0[c] * fanouts[c], rounded once as the mul.f32 would round it
+                        x = F();
+                        line("selp.f32 " + x + ", " + fhex(t * m.fan[nd.fan_off + c]) + ", " + fhex(t) + ", " + pfb + ";");
+                    } else {
+                        x = F();
+                        line("mul.f32 " + x + ", " + lam[c] + ", " + fhex(t) + ";");
+                    }
                 }
             } else {
                 for (int p = 0; p < cols; ++p) {
@@ -259,6 +270,8 @@ struct Gen {
                 }
                 if (!x.empty() && !lam.empty()) line("mul.f32 " + x + ", " + x + ", " + lam[c] + ";");
             }
+            if (fan && !x.empty() && !(root && lam.empty()))
+                line("@" + pfb + " mul.f32 " + x + ", " + x + ", " + fhex(m.fan[nd.fan_off + c]) + ";");
             if (x.empty()) {   // an all-zero CPT row: the state holds no mass
                 if (zero.empty()) { zero = F(); line("mov.f32 " + zero + ", 0f00000000;"); }
                 pi[c] = zero;
@@ -428,10 +441,12 @@ std::string gen_kernel(const bc_model& m, bool dense, int threads, int min_block
 // The marginal of `target`: the upward pass of every subtree off the root -> target path (Gen::message), then the downward
 // chain of path_step, then card(target) stores per query.
 std::string gen_marginal_kernel(const bc_model& m, int target, bool dense, int threads, int min_blocks, long long* n_fma) {
-    Gen g(m, dense, false);
+    Gen g(m, dense);
     g.sync_every = env_int("BC_SPEC_SYNC_EVERY", 0);
     if (!dense)
         for (int w = 0; w < m.bits_words; ++w) g.words.push_back(g.R());
+    if (g.any_fan)   // (a model without fan-out vectors gets the same registers, and the same source, as without a mask)
+        for (int w = 0; w < m.mask_words; ++w) g.fmw.push_back(g.R());
     std::vector<int> path;
     for (int v = target; v > 0; v = m.nodes[v].parent) path.push_back(v);
     path.push_back(0);

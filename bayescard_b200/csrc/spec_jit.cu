@@ -198,7 +198,8 @@ bool bc_marg_attached(bc_model* m, int target) {
     return !m->marg.empty() && m->marg[target].lib != nullptr;
 }
 
-int bc_marg_launch(bc_model* m, const void* desc, size_t nq, int fmt, int target, float* out, cudaStream_t stream) {
+int bc_marg_launch(bc_model* m, const void* desc, size_t nq, int fmt, const uint32_t* fan_mask, int target, float* out,
+                   cudaStream_t stream) {
     BcMargSlot s;
     {
         std::lock_guard<std::mutex> lock(m->marg_mu);
@@ -213,9 +214,8 @@ int bc_marg_launch(bc_model* m, const void* desc, size_t nq, int fmt, int target
     const unsigned char* d = static_cast<const unsigned char*>(desc);
     unsigned long long stride = (unsigned long long)bc_model_desc_stride(m, fmt);
     unsigned long long n = nq;
-    const uint32_t* no_mask = nullptr;
     uint64_t* ctr = m->d_spec_ctr + 2 * (m->spec_ctr_next.fetch_add(1) % BC_SPEC_CTR_SLOTS);
-    void* args[] = {(void*)&d, (void*)&stride, (void*)&no_mask, (void*)&out, (void*)&n, (void*)&ctr};
+    void* args[] = {(void*)&d, (void*)&stride, (void*)&fan_mask, (void*)&out, (void*)&n, (void*)&ctr};
     const int resident = fmt == BC_DESC_DENSE_F32 ? s.blocks_dense : s.blocks_bits;
     long long grid = (long long)m->sm_count * resident;
     const long long needed = (long long)((nq + s.threads - 1) / s.threads);

@@ -143,31 +143,40 @@ class DeviceModel:
         return int(L.lib().bc_model_marginal_hash(self._h, self._check_node(node)))
 
     def run_marginal_device(self, desc_ptr: int, n: int, fmt: int, node: int, out_ptr: int, kernel: int = L.KERNEL_AUTO,
-                            stream: int = 0) -> None:
-        """``bc_marginal_batch`` on DEVICE buffers: ``out`` receives ``[n][card(node)]`` fp32."""
-        L.check(L.lib().bc_marginal_batch(self._h, desc_ptr or None, n, fmt, int(node), out_ptr or None, kernel, stream or None))
+                            stream: int = 0, mask_ptr: int = 0) -> None:
+        """``bc_expectation_marginal_batch`` on DEVICE buffers: ``out`` receives ``[n][card(node)]`` fp32; ``mask_ptr``: 0 or
+        ``n * mask_words`` uint32 fan-out mask rows (0 is ``bc_marginal_batch``)."""
+        L.check(L.lib().bc_expectation_marginal_batch(self._h, desc_ptr or None, n, fmt, mask_ptr or None, int(node), out_ptr or None,
+                                                      kernel, stream or None))
 
-    def run_marginal_host(self, desc: np.ndarray, fmt: int, node: int, kernel: int = L.KERNEL_AUTO) -> np.ndarray:
+    def run_marginal_host(self, desc: np.ndarray, fmt: int, node: int, kernel: int = L.KERNEL_AUTO,
+                          mask: Optional[np.ndarray] = None) -> np.ndarray:
         """BITS / DENSE_F32 rows from the host -> ``ndarray [n, card(node)]`` fp32: the per-state mass of ``node`` under
-        each row.  torch moves the buffers; the work is ``bc_marginal_batch``."""
+        each row, with the fan-out columns of ``mask`` (``[n, mask_words]`` uint32, or ``None``) multiplied in.  torch moves
+        the buffers; the work is ``bc_expectation_marginal_batch``."""
         node = self._check_node(node)
         stride = self.desc_stride(fmt)
         desc = np.ascontiguousarray(desc)
         n = desc.nbytes // stride
         if desc.nbytes != n * stride:
             raise ValueError(f"descriptor buffer of {desc.nbytes} B is not a multiple of the row stride {stride}")
+        if mask is not None:
+            mask = np.ascontiguousarray(mask, dtype=np.uint32)
+            if mask.size != n * self.mask_words:
+                raise ValueError("fan-out mask has the wrong size")
         card = int(self.tm.card[node])
         if n == 0 or self.device < 0:   # (the library still validates the arguments)
-            L.check(L.lib().bc_marginal_batch(self._h, None, n, fmt, node, None, kernel, None))
+            L.check(L.lib().bc_expectation_marginal_batch(self._h, None, n, fmt, None, node, None, kernel, None))
             return np.zeros((n, card), dtype=np.float32)
         import torch
 
         dev = torch.device("cuda", self.device)
         with torch.cuda.device(dev):
             d_desc = torch.from_numpy(desc.reshape(-1).view(np.uint8)).to(dev)
+            d_mask = torch.from_numpy(mask.reshape(-1)).to(dev) if mask is not None else None
             d_out = torch.empty(n * card, dtype=torch.float32, device=dev)
             self.run_marginal_device(d_desc.data_ptr(), n, fmt, node, d_out.data_ptr(), kernel,
-                                     torch.cuda.current_stream().cuda_stream)
+                                     torch.cuda.current_stream().cuda_stream, d_mask.data_ptr() if d_mask is not None else 0)
             return d_out.cpu().numpy().reshape(n, card)
 
     # ------------------------------------------------------------------ geometry

@@ -69,10 +69,12 @@ class VariableEliminationB200:
                 out[i] = 0.0
         return out
 
-    def marginal_batch(self, decoded, name: str, kernel: Optional[int] = None) -> np.ndarray:
+    def marginal_batch(self, decoded, name: str, kernel: Optional[int] = None,
+                       fanouts: Optional[Sequence[Sequence[str]]] = None) -> np.ndarray:
         """GROUP BY ``name``: ``[len(decoded), card]`` fp64, row i = the per-state mass of column ``name`` under the
-        already decoded query i (``bc_marginal_batch``; its row sums are what ``run_decoded`` returns).  The first call for
-        a column attaches its specialised marginal kernel; a sharded machine answers on its first replica."""
+        already decoded query i, weighted by the fan-out columns ``fanouts[i]`` when given (``bc_expectation_marginal_batch``;
+        its row sums are what ``run_decoded(decoded, fanouts)`` returns).  The first call for a column attaches its
+        specialised marginal kernel; a sharded machine answers on its first replica."""
         v = self.tm._index[name]
         kernel = self.kernel if kernel is None else kernel
         dm = self._single
@@ -81,11 +83,11 @@ class VariableEliminationB200:
         out = np.zeros((len(decoded), int(self.tm.card[v])), dtype=np.float64)
         if len(decoded) == 0:
             return out
-        b_idx, b_desc, d_idx, d_desc, _ = self.compiler.pack(decoded)
+        b_idx, b_desc, d_idx, d_desc, mask = self.compiler.pack(decoded, fanouts)
         if len(b_idx):
-            out[b_idx] = dm.run_marginal_host(b_desc, L.DESC_BITS, v, kernel)
+            out[b_idx] = dm.run_marginal_host(b_desc, L.DESC_BITS, v, kernel, None if mask is None else mask[b_idx])
         if len(d_idx):
-            out[d_idx] = dm.run_marginal_host(d_desc, L.DESC_DENSE_F32, v, kernel)
+            out[d_idx] = dm.run_marginal_host(d_desc, L.DESC_DENSE_F32, v, kernel, None if mask is None else mask[d_idx])
         return out
 
     @staticmethod

@@ -135,6 +135,10 @@ def _first_table(order: Sequence[str], conds: Dict[str, list]) -> str:
 def plan_star_query(sql: str, join_sizes: Dict[int, float]) -> list:
     """One job-light SQL text -> ``[full_join_size, factor, ...]`` in the reference's format."""
     order, conds = parse_job_light(sql)
+    return _plan(order, conds, join_sizes)
+
+
+def _plan(order: Sequence[str], conds: Dict[str, list], join_sizes: Dict[int, float]) -> list:
     if not order:
         raise ValueError("no joined table")
     c_t = _table_query("title", conds.get("title", []))
@@ -166,6 +170,82 @@ def plan_star_query(sql: str, join_sizes: Dict[int, float]) -> list:
 
 def plan_workload(sqls: Sequence[str], join_sizes: Dict[int, float]) -> List[list]:
     return [plan_star_query(s, join_sizes) for s in sqls]
+
+
+# ------------------------------------------------------------------------------------ GROUP BY over the star
+class _GroupValue:
+    """The placeholder of the grouping column's value in a planned GROUP BY (kept as one object through deep copies)."""
+
+    def __repr__(self):
+        return "GROUP_VALUE"
+
+    def __copy__(self):
+        return self
+
+    def __deepcopy__(self, memo):
+        return self
+
+
+GROUP_VALUE = _GroupValue()
+
+
+def parse_job_light_groupby(sql: str) -> Tuple[List[str], Dict[str, List[Tuple[str, str, float]]], str, str]:
+    """``SELECT x.col, COUNT(*) FROM ... WHERE ... GROUP BY x.col`` (job-light's grammar otherwise) -> (joined tables, conditions
+    as :func:`parse_job_light` returns them, grouping table, grouping column)."""
+    sql = sql.strip().rstrip(";").strip()
+    m = re.match(r"(?is)^select\s+(.*?)\s+from\s+(.*?)\s+group\s+by\s+(\w+)\.(\w+)$", sql)
+    if not m:
+        raise ValueError("not a job-light GROUP BY query: " + sql[:80])
+    items = [x.strip() for x in m.group(1).split(",")]
+    galias, gcol = m.group(3), m.group(4)
+    if sorted(x.lower().replace(" ", "") for x in items) != sorted(["count(*)", f"{galias}.{gcol}".lower()]):
+        raise ValueError("the select list of a GROUP BY must be the grouping column and COUNT(*): " + m.group(1))
+    rest = m.group(2)
+    order, conds = parse_job_light("SELECT COUNT(*) FROM " + rest)
+    alias_of = {part.split()[-1]: part.split()[0] for part in re.split(r"(?i)\s+where\s+", rest)[0].split(",")}
+    if galias not in alias_of:
+        raise ValueError(f"grouping column {galias}.{gcol}: unknown alias")
+    return order, conds, alias_of[galias], gcol
+
+
+def plan_star_groupby(sql: str, join_sizes: Dict[int, float]) -> dict:
+    """One job-light GROUP BY text -> ``{"column", "where", "plan"}``, the plan of every group at once.
+
+    ``plan`` is :func:`plan_star_query`'s factor list for the query with the grouping column counted as a conditioned column:
+    an equality with the placeholder :data:`GROUP_VALUE`, which is what the per-value query ``... AND x.col = v`` sees (``=``
+    wins over the column's other conditions in ``_table_query``).  ``_first_table``, ``factor_refine`` and the title conditions
+    therefore do not depend on v: :func:`groupby_value_plan` with v is ``plan_star_query`` of the per-value text.  ``where`` is
+    the ``_table_query`` value of the grouping column's own WHERE conditions (``None`` without any): they select the groups."""
+    order, conds, table, col = parse_job_light_groupby(sql)
+    where = _table_query(table, [c for c in conds.get(table, []) if c[0] == col]).get(f"{table}.{col}")
+    conds = {t: list(c) for t, c in conds.items()}
+    conds.setdefault(table, []).append((col, "=", GROUP_VALUE))
+    return {"column": f"{table}.{col}", "where": where, "plan": _plan(order, conds, join_sizes)}
+
+
+def groupby_value_plan(planned: dict, value) -> list:
+    """The plan of one group: ``planned["plan"]`` with the placeholder replaced by ``value``."""
+    out = [planned["plan"][0]]
+    for f in planned["plan"][1:]:
+        q = {k: (value if x is GROUP_VALUE else x) for k, x in f["query"].items()}
+        out.append({"bn_index": f["bn_index"], "inverse": f["inverse"], "query": q, "expectation": list(f["expectation"])})
+    return out
+
+
+def groupby_sql_batch(ensemble, sqls: Sequence[str], join_sizes: Dict[int, float] = None) -> List[dict]:
+    """job-light GROUP BY texts -> one ``{key: estimate}`` per text (:meth:`BN_ensemble.groupby_batch`; the texts that group
+    by the same column are answered together).  ``join_sizes``: ``{bn_index: full join size}``, by default each BN's
+    ``nrows``."""
+    if join_sizes is None:
+        join_sizes = {i: float(ensemble.bns[i].nrows) for i in range(len(BN_INDEX))}
+    planned = [plan_star_groupby(s, join_sizes) for s in sqls]
+    out: List[dict] = [{} for _ in sqls]
+    for column in dict.fromkeys(p["column"] for p in planned):
+        idx = [i for i, p in enumerate(planned) if p["column"] == column]
+        keys, est = ensemble.groupby_batch([planned[i] for i in idx], column)
+        for j, i in enumerate(idx):
+            out[i] = {k: float(e) for k, e in zip(keys, est[j])}
+    return out
 
 
 class NativeJobLight:

@@ -6,7 +6,8 @@ Mirrors the public surface of the reference class for the exact-jit path
 metadata attributes drivers read (``nrows``, ``attr_type``, ``domain``, ``encoding``, ``fanouts``, ...).
 Only ``infer_algo='exact-jit'`` exists here; the other algorithms of the reference are out of scope.
 
-New next to the scalar methods: ``query_batch`` / ``expectation_batch`` (one CUDA launch per batch).
+New next to the scalar methods: ``query_batch`` / ``expectation_batch`` (one CUDA launch per batch) and the GROUP BY
+forms ``groupby_batch`` / ``expectation_groupby_batch`` (one pass per query for every group).
 """
 from __future__ import annotations
 
@@ -182,6 +183,24 @@ class Bayescard_BN:
           ``mapping``); the predicate on ``column`` stays, with its coverage weights, and ``est(b) = nrows * M[b]``.
 
         Undecodable queries give a zero row; a query without predicates gives the column's marginal."""
+        return self._groupby(queries, None, column, return_prob)
+
+    def expectation_groupby_batch(self, queries: Sequence[dict], fanout_attrs: Sequence[Sequence[str]], column: str,
+                                  return_prob: bool = False):
+        """:meth:`groupby_batch` of an expectation: query i is weighted by its fan-out columns ``fanout_attrs[i]``, so that
+        ``est[i, j]`` is ``self.expectation({**P_without_column, column: keys[j]}, fanout_attrs[i])`` for the values the
+        predicate on ``column`` selects (0 for the others) -- the factor of a join estimate for every group at once, one
+        pass per query (``bc_expectation_marginal_batch``).  Keys and value selection are those of :meth:`groupby_batch`.
+        Undecodable queries give a zero row (where ``expectation`` raises ``AttributeError``).  Grouping by a fan-out column
+        raises ``ValueError``."""
+        v = self.tree._index.get(column)
+        if column in self.fanout_attr or (v is not None and self.tree.fan_vector(v) is not None):
+            raise ValueError(f"column {column!r} is a fan-out column; GROUP BY needs a column of the table")
+        if len(fanout_attrs) != len(queries):
+            raise ValueError("one list of fan-out columns per query")
+        return self._groupby(queries, [list(f or []) for f in fanout_attrs], column, return_prob)
+
+    def _groupby(self, queries, fanout_attrs, column, return_prob):
         m = self._machine()
         v = self.tree._index.get(column)
         if v is None:
@@ -215,7 +234,7 @@ class Bayescard_BN:
             decoded.append((b, w))
             keep.append(i)
         if decoded:
-            M = m.marginal_batch(decoded, column)
+            M = m.marginal_batch(decoded, column, fanouts=None if fanout_attrs is None else [fanout_attrs[i] for i in keep])
             if categorical:
                 est[keep] = M[:, key_bin] * key_wt[None, :] * np.asarray(sel)
             else:

@@ -169,7 +169,8 @@ BC_API int bc_query_batch_host(bc_model* m, const void* desc, size_t n_queries, 
  * with ONE pass per query: for the target node t (topological index) and each row's weights w_v,
  *     out[q][b] = sum_{x : x_t = b} prod_v w_v[x_v] T_v[x_v, x_pa(v)]          b = 0 .. card(t) - 1
  * so w_t restricts the groups and sum_b out[q][b] is the out_prob[q] of bc_query_batch on the same row.  out is contiguous
- * fp32 [n_queries][card(t)].  Rows are BITS or DENSE_F32; there is no fan-out mask (fan-out columns are unconstrained).
+ * fp32 [n_queries][card(t)].  Rows are BITS or DENSE_F32; there is no fan-out mask (fan-out columns are unconstrained:
+ * bc_expectation_marginal_batch below with a NULL mask, which is what this call is).
  * DEVICE pointers, stream ordered.  kernel:
  *   BC_KERNEL_AUTO   the specialised marginal kernel of t when it is attached, otherwise the expansion below
  *   BC_KERNEL_SPEC   the specialised marginal kernel of t; BC_ECOMPILE when it is not attached
@@ -179,6 +180,17 @@ BC_API int bc_query_batch_host(bc_model* m, const void* desc, size_t n_queries, 
  * with no launch.  Results below the fp32 range are not carried (no scaled form). */
 BC_API int bc_marginal_batch(bc_model* m, const void* desc, size_t n_queries, int desc_format, int target, float* out,
                              int kernel, void* stream);
+/* GROUP BY one column of an EXPECTATION: replaces `[bn.expectation({**P, a: v}, fan) for v in values]` over
+ * Bayescard_BN.expectation (Models/Bayescard_BN.py:559) -- the per-value loop of a GROUP BY over a join, where every factor
+ * is weighted by fan-out columns -- with ONE pass per query.  fanout_mask has bc_query_batch's layout and meaning: NULL or
+ * n_queries * mask_words uint32, bit v of row q multiplies w_v by fanouts[v] (w'_v), and
+ *     out[q][b] = sum_{x : x_t = b} prod_v w'_v[x_v] T_v[x_v, x_pa(v)]
+ * so sum_b out[q][b] is bc_query_batch's out_prob[q] on the same row and mask.  Formats, kernel ids, argument checks and
+ * error codes are bc_marginal_batch's; a NULL mask is exactly bc_marginal_batch.  The specialised marginal kernel reads the
+ * mask in place (still one launch); the expansion repeats each mask row card(t) times next to the expanded rows (counted
+ * in the 256 MB chunk bound) and passes it to bc_query_batch. */
+BC_API int bc_expectation_marginal_batch(bc_model* m, const void* desc, size_t n_queries, int desc_format,
+                                         const uint32_t* fanout_mask, int target, float* out, int kernel, void* stream);
 /* Build (or load "<cache_dir>/marg_<hash>.cubin") the specialised marginal kernel of one target node: straight-line sm_100a
  * code like bc_model_specialize's, attached through the driver JIT; one module per target, kept on the model. */
 BC_API int bc_model_specialize_marginal(bc_model* m, int target, const char* cache_dir);
