@@ -124,6 +124,11 @@ _SIGS = {
                                   C.c_void_p, C.POINTER(C.c_size_t)]),
     "bc_fit_counts": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_size_t,
                                 C.c_void_p, C.c_size_t, C.POINTER(C.c_uint32), C.c_void_p]),
+    "bc_model_set_counts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),
+    "bc_model_get_counts": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "bc_model_arena": (C.c_int64, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]),
+    "bc_model_update": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_int, C.c_size_t, C.c_void_p,
+                                  C.POINTER(C.c_uint32), C.c_void_p]),
     "bc_pair_counts": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_size_t, C.c_void_p,
                                  C.c_size_t, C.POINTER(C.c_uint32), C.c_void_p]),
     "bc_chow_liu": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_void_p,

@@ -67,6 +67,11 @@ static int pipe_quiesce(BcHostPipe* p) {
     return BC_OK;
 }
 
+int bc_pipe_quiesce_model(bc_model* m) {
+    std::lock_guard<std::mutex> lock(m->pipe_mu);
+    return pipe_quiesce(m->pipe);
+}
+
 static void pipe_free(BcHostPipe* p) {
     if (!p) return;
     for (int i = 0; i < BcHostPipe::kSlots; ++i) {
@@ -262,8 +267,26 @@ extern "C" void bc_model_destroy(bc_model* m) {
         cudaFree(m->d_dense_default);
         cudaFree(m->d_spec_ctr);
         cudaFree(m->d_ent_node);
+        cudaFree(m->d_counts);
+        cudaFree(m->d_upd);
     }
     delete m;
+}
+
+void bc_model_drop_cached(bc_model* m) {
+    if (m->spec_lib) cudaLibraryUnload(m->spec_lib);
+    m->spec_lib = nullptr;
+    m->spec_range8 = m->spec_dense = m->spec_bits = nullptr;
+    {
+        std::lock_guard<std::mutex> lock(m->marg_mu);
+        bc_marg_free(m);
+    }
+    {
+        std::lock_guard<std::mutex> lock(m->k2_mu);
+        bc_k2_free(m);
+    }
+    std::lock_guard<std::mutex> lock(m->k3_mu);
+    bc_k3_free(m);
 }
 
 extern "C" int bc_model_n_nodes(const bc_model* m) { return m ? m->n : 0; }
@@ -293,6 +316,20 @@ extern "C" int bc_model_bits_default(const bc_model* m, void* row_host, size_t r
     return BC_OK;
 }
 extern "C" int64_t bc_model_flops_dense(const bc_model* m) { return m ? m->flops_dense : 0; }
+extern "C" int64_t bc_model_arena(const bc_model* m, int from_device, float* out, size_t capacity) {
+    if (!m) { bc_set_error("model is NULL"); return BC_EINVAL; }
+    const size_t floats = m->arena_floats_padded;
+    if (!out || capacity < floats) return (int64_t)floats;
+    if (!from_device) {
+        if (m->arena.empty()) { bc_set_error("the model keeps no host copy of its arena"); return BC_ELIMIT; }
+        std::memcpy(out, m->arena.data(), floats * sizeof(float));
+        return (int64_t)floats;
+    }
+    if (m->device < 0) { bc_set_error("model has no device (host-only model)"); return BC_EINVAL; }
+    BC_CUDA_CHECK(cudaSetDevice(m->device));
+    BC_CUDA_CHECK(cudaMemcpy(out, m->d_arena, floats * sizeof(float), cudaMemcpyDeviceToHost));
+    return (int64_t)floats;
+}
 extern "C" int bc_model_has_spec(const bc_model* m) {
     return m && (m->spec_range8 || m->spec_bits || m->spec_dense) ? 1 : 0;
 }

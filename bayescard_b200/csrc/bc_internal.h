@@ -107,10 +107,20 @@ struct bc_model {
     std::mutex k3_mu;
     BcHostPipe* pipe = nullptr;
     std::mutex pipe_mu;
+    // counts behind the CPTs (bc_model_set_counts / bc_model_update, bc_fit.cu): bc_fit_counts' layout, node v's counters
+    // from cnt_off[v], its columns (one per parent state) from col_off[v]; both arrays end with the total
+    unsigned long long* d_counts = nullptr;
+    void* d_upd = nullptr;           // per-node table of the update kernels
+    std::vector<int64_t> cnt_off, col_off;
+    bool has_counts = false;
 };
 
 void bc_set_error(const char* fmt, ...);
 void bc_count_launch(uint64_t n = 1);
+// bc_api.cu: wait for the model's asynchronous host submissions; drop everything built from the CPT values (spec and
+// marginal modules, K2 and K3 plans), which the next use rebuilds
+int bc_pipe_quiesce_model(bc_model* m);
+void bc_model_drop_cached(bc_model* m);
 
 #define BC_CUDA_CHECK(expr)                                                                      \
     do {                                                                                         \

@@ -47,6 +47,8 @@ class DeviceModel:
         self.spec_error: Optional[str] = None
         self.marginal_error: Dict[int, str] = {}   # target node -> why its specialised marginal kernel is missing
         self._marginal_built: Dict[int, bool] = {}
+        self._specialize = specialize and device >= 0   # update() re-specialises under the same policy
+        self._cache_dir = cache_dir
         if specialize and device >= 0:
             try:
                 self.specialize(cache_dir)
@@ -178,6 +180,97 @@ class DeviceModel:
             self.run_marginal_device(d_desc.data_ptr(), n, fmt, node, d_out.data_ptr(), kernel,
                                      torch.cuda.current_stream().cuda_stream, d_mask.data_ptr() if d_mask is not None else 0)
             return d_out.cpu().numpy().reshape(n, card)
+
+    # ------------------------------------------------------------------ incremental update (DESIGN.md section 9e)
+    def attach_counts(self, counts: np.ndarray) -> None:
+        """Keep ``counts`` (uint64, ``fit.count_layout`` order) on the device as the counts behind the CPTs
+        (``bc_model_set_counts``).  They must be the counts the CPTs were normalised from (``fit.counts_from_cpts``)."""
+        counts = np.ascontiguousarray(counts, dtype=np.uint64)
+        L.check(L.lib().bc_model_set_counts(self._h, counts.ctypes.data, counts.size))
+        self._marginal_built.clear()
+        self.marginal_error.clear()
+
+    def get_counts(self, node_first: int = 0, node_count: Optional[int] = None) -> np.ndarray:
+        """The attached counters of nodes ``[node_first, node_first + node_count)`` (default: to the last node)."""
+        from .fit import count_layout
+
+        node_count = self.n_nodes - node_first if node_count is None else node_count
+        off, total = count_layout(self.tm.parent, self.tm.card)
+        off = np.append(off, total)
+        if not (0 <= node_first and 0 <= node_count and node_first + node_count <= self.n_nodes):
+            raise ValueError(f"nodes [{node_first}, {node_first + node_count}) outside the model's {self.n_nodes} nodes")
+        out = np.zeros(int(off[node_first + node_count] - off[node_first]), dtype=np.uint64)
+        L.check(L.lib().bc_model_get_counts(self._h, node_first, node_count, out.ctypes.data if out.size else None))
+        return out
+
+    def arena(self, from_device: bool = True) -> np.ndarray:
+        """The fp32 CPT arena the kernels read (``from_device``) or the library's host copy of it, zero-padded: its first
+        ``tm.pack_arena()[0].size`` floats are ``pack_arena()``'s."""
+        lib = L.lib()
+        n = int(lib.bc_model_arena(self._h, int(from_device), None, 0))
+        if n < 0:
+            L.check(n)
+        out = np.zeros(n, dtype=np.float32)
+        rc = int(lib.bc_model_arena(self._h, int(from_device), out.ctypes.data, n))
+        if rc < 0:
+            L.check(rc)
+        return out
+
+    def update(self, inserted=None, deleted=None, n_inserted: int = 0, n_deleted: int = 0, elem_bytes: int = 1,
+               row_stride: Optional[int] = None, stream: int = 0) -> np.ndarray:
+        """Insert and delete rows of the table the attached counts came from (``bc_model_update``) and return the
+        topological indices of the nodes whose counts changed.
+
+        Rows are bin ids with columns in topological order.  Either host arrays (``[n, n_nodes]`` or wider, uint8 /
+        uint16; the two tables are given the same width and dtype) or DEVICE addresses with ``n_inserted`` /
+        ``n_deleted`` rows, ``elem_bytes`` and ``row_stride`` (elements, default ``n_nodes``) on ``stream``.  Only the CPTs
+        move: the tree, the decode metadata and the fan-out vectors stay.  A rejected batch (a bin id outside its domain, a
+        delete below zero) raises and leaves the model as it was.  When a count changed, the marginal kernels are
+        forgotten and, for a model built with ``specialize=True``, the specialised kernel is built again for the new
+        CPTs."""
+        host = not (isinstance(inserted, int) or isinstance(deleted, int))
+        touched = np.zeros(self.n_nodes, dtype=np.uint8)
+        bad = C.c_uint32(0)
+        if host:
+            tabs = [None if t is None else np.asarray(t) for t in (inserted, deleted)]
+            present = [t for t in tabs if t is not None]
+            for t in present:
+                if t.ndim != 2 or t.shape[1] < self.n_nodes or t.dtype not in (np.uint8, np.uint16):
+                    raise ValueError("rows must be [n, >= n_nodes] uint8 or uint16 bin ids")
+            dt = np.uint16 if any(t.dtype == np.uint16 for t in present) else np.uint8
+            width = max([t.shape[1] for t in present], default=self.n_nodes)
+            tabs = [None if t is None else
+                    np.ascontiguousarray((t if t.shape[1] == width else np.pad(t, ((0, 0), (0, width - t.shape[1])))).astype(dt, copy=False))
+                    for t in tabs]
+            n_ins, n_del = [0 if t is None else t.shape[0] for t in tabs]
+            if n_ins + n_del and self.device >= 0:
+                import torch
+
+                dev = torch.device("cuda", self.device)
+                with torch.cuda.device(dev):
+                    d = [None if not (t is not None and t.shape[0]) else torch.from_numpy(t.reshape(-1).view(np.uint8)).to(dev)
+                         for t in tabs]
+                    L.check(L.lib().bc_model_update(self._h, d[0].data_ptr() if d[0] is not None else None, n_ins,
+                                                    d[1].data_ptr() if d[1] is not None else None, n_del, np.dtype(dt).itemsize,
+                                                    width, touched.ctypes.data, C.byref(bad), torch.cuda.current_stream().cuda_stream or None))
+            else:   # (no rows, or a host-only model: the library still validates the arguments)
+                L.check(L.lib().bc_model_update(self._h, None, 0, None, 0, np.dtype(dt).itemsize, width, touched.ctypes.data,
+                                                C.byref(bad), None))
+        else:
+            L.check(L.lib().bc_model_update(self._h, inserted or None, n_inserted, deleted or None, n_deleted, elem_bytes,
+                                            self.n_nodes if row_stride is None else row_stride, touched.ctypes.data, C.byref(bad),
+                                            stream or None))
+        nodes = np.flatnonzero(touched)
+        if nodes.size:
+            self._marginal_built.clear()
+            self.marginal_error.clear()
+            if self._specialize:
+                try:
+                    self.specialize(self._cache_dir)
+                    self.spec_error = None
+                except L.BayesCardError as e:
+                    self.spec_error = str(e)
+        return nodes
 
     # ------------------------------------------------------------------ geometry
     def desc_stride(self, fmt: int) -> int:
@@ -502,6 +595,24 @@ class ShardedModel:
     def wait(self, tickets) -> None:
         for rep, t in tickets:
             rep.wait(t)
+
+    def attach_counts(self, counts: np.ndarray) -> None:
+        for r in self.replicas:
+            r.attach_counts(counts)
+
+    def get_counts(self, node_first: int = 0, node_count: Optional[int] = None) -> np.ndarray:
+        return self.replicas[0].get_counts(node_first, node_count)
+
+    def update(self, inserted=None, deleted=None) -> np.ndarray:
+        """The same batch (host arrays, see ``DeviceModel.update``) on every replica, each from its own host thread.
+        Counts are integers and the normalisation is exact, so the replicas stay bit-identical.  Returns the touched
+        nodes."""
+        futs = [self._pool.submit(r.update, inserted, deleted) for r in self.replicas]
+        errs = [f.exception() for f in futs]
+        for e in errs:
+            if e is not None:
+                raise e
+        return futs[0].result()
 
     def close(self):
         self._pool.shutdown(wait=True)

@@ -153,6 +153,11 @@ class TreeModel:
     n_mcv: Any = None
     n_bins: Any = None
     root: Any = None
+    # --- counts behind the CPTs (fit.count_layout order, uint64) and the rows they were counted from; known when the
+    #     CPTs were fitted here (fit.refit, structure.learn_tree_model), recovered by fit.counts_from_cpts otherwise.
+    #     Neither is stored in the .npz / .bcm files: the CPTs determine them.
+    counts: Optional[np.ndarray] = None
+    fit_rows: Optional[int] = None
 
     # ------------------------------------------------------------------ derived
     @property

@@ -6,8 +6,9 @@ Mirrors the public surface of the reference class for the exact-jit path
 metadata attributes drivers read (``nrows``, ``attr_type``, ``domain``, ``encoding``, ``fanouts``, ...).
 Only ``infer_algo='exact-jit'`` exists here; the other algorithms of the reference are out of scope.
 
-New next to the scalar methods: ``query_batch`` / ``expectation_batch`` (one CUDA launch per batch) and the GROUP BY
-forms ``groupby_batch`` / ``expectation_groupby_batch`` (one pass per query for every group).
+New next to the scalar methods: ``query_batch`` / ``expectation_batch`` (one CUDA launch per batch), the GROUP BY
+forms ``groupby_batch`` / ``expectation_groupby_batch`` (one pass per query for every group) and ``update_rows``
+(inserted / deleted rows move the CPTs on the GPU without a refit).
 """
 from __future__ import annotations
 
@@ -260,6 +261,52 @@ class Bayescard_BN:
                 out[i] = {k: float(e) for k, e in zip(keys, est[j])}
         return out
 
+    # ------------------------------------------------------------------ table changes
+    def update_rows(self, inserted=None, deleted=None, fit_rows: Optional[int] = None) -> List[str]:
+        """Follow rows inserted into / deleted from the table without a refit: the CPTs become those of ``fit.refit`` on
+        the rows the model was fitted on plus ``inserted`` minus ``deleted`` (same tree), on the GPU, and ``nrows`` moves by
+        the difference.  Returns the names of the columns whose CPTs changed.
+
+        Rows are bin ids (``[n, len(node_names)]``, uint8 / uint16) with columns in ``node_names`` order -- for
+        ``build_from_table`` the table's own column order; columns in ``dropped_names`` are ignored.  Only the CPTs move:
+        the tree, the discretisation (``encoding``, ``n_in_bin``, ``mapping``, ``domain``) and the fan-out vectors stay as
+        they are.  A model fitted on a sample (``fit_rows < nrows``) counts inserted rows with weight 1 against the
+        sample's counts.  A batch holding an out-of-domain bin id, or deleting more rows of some (column, parent) bin pair
+        than were counted, raises and changes nothing; deleting rows that were never in the data cannot be detected
+        otherwise.
+
+        The first call attaches the counts behind the CPTs: the tree model's own when it has them, otherwise
+        ``fit.counts_from_cpts`` with ``fit_rows`` (default: ``tree.fit_rows``, else ``fit.infer_fit_rows``)."""
+        from .fit import count_layout, counts_from_cpts, infer_fit_rows, node_cpt
+
+        m = self._machine()
+        t = self.tree
+        if not getattr(self, "_counts_attached", False):
+            if t.counts is None:
+                rows = fit_rows if fit_rows is not None else (t.fit_rows if t.fit_rows is not None else infer_fit_rows(t))
+                t.counts = counts_from_cpts(t.parent, t.card, t.cpts, rows)
+                t.fit_rows = int(rows)
+            elif t.fit_rows is None:
+                t.fit_rows = int(np.asarray(t.counts[: int(t.card[0])], dtype=np.uint64).sum())
+            t.counts = np.array(t.counts, dtype=np.uint64)   # (a private, writable copy: refreshed below)
+            m.dev.attach_counts(t.counts)
+            self._counts_attached = True
+        tabs = [None if rows is None else rows_to_topological(t, rows) for rows in (inserted, deleted)]
+        touched = m.dev.update(tabs[0], tabs[1])
+        off, total = count_layout(t.parent, t.card)
+        off = np.append(off, total)
+        for v in touched:   # the host mirror of the touched nodes: counts and fp64 CPTs
+            c = m.dev.get_counts(int(v), 1)
+            t.counts[off[v]: off[v + 1]] = c
+            t.cpts[v] = node_cpt(t.parent, t.card, int(v), c)
+        delta = (0 if tabs[0] is None else tabs[0].shape[0]) - (0 if tabs[1] is None else tabs[1].shape[0])
+        t.fit_rows += delta
+        t.nrows = t.nrows + delta
+        self.nrows = t.nrows
+        if self.cpds is not None:
+            self.cpds = list(t.cpts)
+        return [t.infer_names[int(v)] for v in touched]
+
     def close(self):
         if getattr(self, "_sqlc", None) is not None:
             self._sqlc.close()
@@ -267,6 +314,25 @@ class Bayescard_BN:
         if self.infer_machine is not None:
             self.infer_machine.close()
             self.infer_machine = None
+
+
+def rows_to_topological(tm: TreeModel, rows) -> np.ndarray:
+    """Rows of bin ids with columns in ``node_names`` order -> the same rows with columns in topological order (the
+    convention of ``bc_fit_counts`` / ``bc_model_update``); columns outside the root component (``dropped_names``) are
+    dropped.  uint8 / uint16 rows keep their type unless a domain needs uint16; other integer types are range-checked and
+    narrowed."""
+    rows = np.asarray(rows)
+    if rows.ndim != 2 or rows.shape[1] != len(tm.node_names):
+        raise ValueError(f"rows must be [n, {len(tm.node_names)}] bin ids in node_names order")
+    wide = int(np.max(tm.card)) > 256
+    if rows.dtype not in (np.uint8, np.uint16):
+        if rows.size and (rows.min() < 0 or rows.max() > 65535):
+            raise ValueError("bin ids must lie in [0, 65535]")
+        rows = rows.astype(np.uint16 if wide or (rows.size and rows.max() > 255) else np.uint8)
+    elif wide:
+        rows = rows.astype(np.uint16)
+    cols = [tm.node_names.index(name) for name in tm.infer_names]
+    return np.ascontiguousarray(rows[:, cols])
 
 
 def load_BN_single(path: str, device=0, **kw) -> Bayescard_BN:

@@ -155,4 +155,5 @@ def model_from_counts(parent: Sequence[int], card: Sequence[int], counts: np.nda
         attr_type={k: "categorical" for k in names}, algorithm="chow-liu", topo_names=topo_names, infer_names=topo_names,
         parent=t_parent, card=t_card, cpts=cpts, dropped_names=[],
         encoding={names[i]: {b: b for b in range(int(card[i]))} for i in range(n)},
-        domain={names[i]: list(range(int(card[i]))) for i in range(n)}, root=root)
+        domain={names[i]: list(range(int(card[i]))) for i in range(n)}, root=root,
+        counts=flat, fit_rows=int(flat[: int(t_card[0])].sum()))

@@ -17,7 +17,8 @@
  *   - every function returning int returns BC_OK (0) on success, a negative BC_E* code otherwise;
  *     bc_last_error() then holds a human-readable message (thread local).
  *   - there is NO CPU fallback: if no CUDA device / kernel image is usable the call fails.
- *   - a bc_model is immutable after creation; bc_query_batch* are stream ordered and may be called
+ *   - a bc_model's tree is fixed at creation and its CPTs change only through bc_model_update;
+ *     bc_query_batch* are stream ordered and may be called
  *     concurrently on different models / devices (one host thread per GPU).
  *   - node indices are TOPOLOGICAL (parents before children, node 0 = root), the order of
  *     align_cpds_in_topological() restricted to the root's component.
@@ -343,6 +344,44 @@ BC_API int bc_sqlc_compile(const bc_sqlc* c, size_t n_queries, const char* const
 BC_API int bc_fit_counts(int device, int n_nodes, const int32_t* parent, const int32_t* card, const void* table_dev,
                          int elem_bytes, size_t n_rows, size_t row_stride_elems, unsigned long long* counts_dev,
                          size_t n_counters, uint32_t* bad_rows_host, void* stream);
+
+/* ---- Incremental update of a served model: rows inserted into / deleted from the table -------------------------
+ * Replaces rerunning `self.model.fit(discrete_table)` of build_from_data (Models/Bayescard_BN.py:108-110) on the changed
+ * table.  The tree stays as it is; only the CPTs follow the counts.  A model keeps u64 counts on the device once they are
+ * attached; an update counts its rows into +/-1 deltas, adds them, and normalises again only the CPT columns (node, parent
+ * state) whose counts moved, in fp64 with bc_fit_counts' caller's rule, so that the arena equals a fresh bc_model_create
+ * of the refitted CPTs bit for bit.
+ *
+ * bc_model_set_counts: counts_host holds n_counters u64 counts in bc_fit_counts' layout (node after node, (c, p) at
+ *   off_v + c * card[parent(v)] + p); n_counters must be the tree's total (checked before any device work).  The CPTs are
+ *   NOT derived from them: the caller attaches counts that match the arena (bayescard_b200/fit.py checks this).  Replaces
+ *   counts attached earlier.  Synchronous.
+ * bc_model_get_counts: the counters of nodes [node_first, node_first + node_count) into counts_host.  Synchronous. */
+BC_API int bc_model_set_counts(bc_model* m, const uint64_t* counts_host, size_t n_counters);
+BC_API int bc_model_get_counts(const bc_model* m, int node_first, int node_count, uint64_t* counts_host);
+/* The fp32 CPT arena as the kernels read it (from_device = 1, synchronous) or its host copy (0; BC_ELIMIT for models too large
+ * to keep one): the arena bc_model_create was given, zero-padded.  Returns the number of floats; with out == NULL or a capacity
+ * below that, nothing is copied. */
+BC_API int64_t bc_model_arena(const bc_model* m, int from_device, float* out, size_t capacity);
+/* One batch: ins_dev / del_dev are DEVICE tables of n_ins / n_del rows of bin ids (bc_fit_counts' convention: row-major,
+ * column v = topological node v, elem_bytes 1 (uint8) or 2 (uint16), row stride row_stride_elems >= n_nodes elements).
+ *   - counts become counts + count(ins) - count(del), integer-exact;
+ *   - the call is rejected with BC_EINVAL, and NOTHING on the model changes, when a row of either table holds a bin id
+ *     outside its node's domain (*bad_rows_host = how many) or when a delete would take a count below zero (the error
+ *     names the node, own bin and parent bin); deleting rows that were never counted is only detected through such an
+ *     underflow;
+ *   - the touched CPT columns are re-normalised in the device arena and mirrored into the host copy, so bc_model_spec_hash
+ *     changes with them; then, if any count changed, the specialised and marginal modules are unloaded (has_spec becomes
+ *     0: call bc_model_specialize again) and the K2 / K3 plans are dropped (rebuilt on their next use).  An update with no
+ *     rows, or whose deltas cancel, changes nothing and keeps every module attached;
+ *   - touched_nodes_host (nullable, n_nodes bytes): 1 for every node whose counts changed; bad_rows_host nullable.
+ * Stream ordered on `stream`: query batches enqueued on it before the call see the old CPTs, those enqueued after it the new
+ * ones (the call synchronises the stream twice: once to validate, once when the host copy of the arena is complete).  No
+ * call on the same model may run concurrently from another stream or host thread.
+ * BC_EINVAL before any device work for: an element size other than 1 / 2, a short row stride, NULL rows, a node whose
+ * card does not fit the element type, or a model without counts. */
+BC_API int bc_model_update(bc_model* m, const void* ins_dev, size_t n_ins, const void* del_dev, size_t n_del, int elem_bytes,
+                           size_t row_stride_elems, uint8_t* touched_nodes_host, uint32_t* bad_rows_host, void* stream);
 
 /* ---- Structure learning: all-pairs counts, mutual information, Chow-Liu tree ------------------------------------
  * Replaces pomegranate's BayesianNetwork.from_samples(algorithm='chow-liu', root=0) (Models/BN_single_model.py:141-202).
