@@ -98,6 +98,12 @@ namespace {
 
 constexpr int kTile = 128;     // queries per CTA tile = TMEM lanes = UMMA M
 constexpr int kMaxEdges = 127; // trees of up to 128 columns
+// Longest contraction an edge may have (states of its child column).  All k-steps of an edge (three TF32 products per 8 states)
+// accumulate into ONE fp32 accumulator in tensor memory, and the error grows with the number of chained accumulations (as in
+// K2, see UmmaCfg in k2_umma.cu): 229-256-state columns (96 chained MMAs) came out up to 1.6e-5 off the fp64 oracle on DENSE
+// rows with fan-out columns, beyond the 1e-5 the kernels are held to.  Columns of <= 128 states (48 MMAs; the shipped models
+// have <= 84) stay within it.
+constexpr int kMaxK = 128;
 constexpr int kBK = 32;        // child states per ring step: one 128-byte row of T_v^T / of the weight box (128-byte swizzle), 4 k-steps of 8
 constexpr int kStagesW = 8;    // DENSE weight ring: at most this many slots of 16 KB (K3Params::w_stages are used; the loads come from HBM)
 constexpr int kWBytes = kTile * kBK * 4;
@@ -637,23 +643,21 @@ __global__ void __launch_bounds__(kThreads, 1) k3_kernel(const __grid_constant__
                     // States >= K of the last block: their rows of T_v^T are zeros in the operand image and whole k-steps past K are not
                     // issued, so any FINITE value there contributes 0 -- BITS rows (bits past the domain are cleared, the message's
                     // padding columns hold the zeros the epilogue wrote) need no masking at all.  In a DENSE row the floats past the
-                    // domain are the column's own pad floats (caller-owned: could be NaN / Inf), then the NEXT column's weights (if
-                    // those are not finite the query's result is not finite anyway) and, past the row, the zeros TMA fills in.
+                    // domain are the column's own pad floats, then the NEXT columns' weights AND pad floats, all of them up to the end
+                    // of the last issued 8-state k-step: the pad floats are caller-owned (could be NaN / Inf, and NaN * 0 is NaN), so
+                    // states K .. round_up(K, 8) - 1 are zeroed.  Past that k-step nothing is read; past the row TMA fills zeros.
                     // (The first version's compare + select over all 32 states was 7.5 % of the instructions of this issue-bound
                     // kernel: ncu, profiles/r2_ncu_36_k3_bits_imdb1.json.)
-                    if (FMT == BC_DESC_DENSE_F32 && (K & 3) != 0 && c0 + kBK > K) {
-                        // only the column's own pad floats (a column occupies round_up(card, 4) floats of the row) can hold anything
-                        // the caller did not mean: one float4 group, picked by a uniform switch
-                        const int r = K - c0, k = r & 3;   // first state past the domain, 1 <= k <= 3 inside its group
+                    if (FMT == BC_DESC_DENSE_F32 && (K & 7) != 0 && c0 + kBK > K) {
+                        // one 8-state group, picked by a uniform switch
+                        const int r = K - c0;   // first state past the domain
 #define K3_MASK_GROUP(G)                                              \
     case G:                                                           \
-        if (k <= 1) u[4 * G + 1] = 0.f;                               \
-        if (k <= 2) u[4 * G + 2] = 0.f;                               \
-        u[4 * G + 3] = 0.f;                                           \
+        _Pragma("unroll") for (int j = 8 * G + 1; j < 8 * G + 8; ++j) \
+            if (j >= r) u[j] = 0.f;                                   \
         break;
-                        switch (r >> 2) {
+                        switch (r >> 3) {
                             K3_MASK_GROUP(0) K3_MASK_GROUP(1) K3_MASK_GROUP(2) K3_MASK_GROUP(3)
-                            K3_MASK_GROUP(4) K3_MASK_GROUP(5) K3_MASK_GROUP(6) K3_MASK_GROUP(7)
                             default: break;
                         }
 #undef K3_MASK_GROUP
@@ -1205,6 +1209,10 @@ int k3_prepare(bc_model* m) {
     if (const char* e = std::getenv("BC_K3_BSTAGES")) b_stages = std::max(2, std::min(kMaxStages, std::atoi(e)));
     while (b_stages > 1 && (size_t)b_stages * npad_max * 256 + fixed > smem_optin) --b_stages;
     if ((size_t)b_stages * npad_max * 256 + fixed > smem_optin || b_stages < 2) return fail("operand rings exceed shared memory");
+    // (after the structural limits: a model that does not fit at all is declined for that reason)
+    for (int v = 1; v < n; ++v)
+        if (m->nodes[v].card > kMaxK)
+            return fail("a non-root column of more than 128 states (one accumulator over its k-steps loses the 1e-5 accuracy)");
     k->b_stages = b_stages;
     k->w_stages = w_stages;
     k->smem = (size_t)b_stages * npad_max * 256 + fixed;

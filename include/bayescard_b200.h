@@ -87,8 +87,8 @@ extern "C" {
                                 where the edge shape allows, FP32 SIMT GEMM otherwise; RANGE_* rows */
 #define BC_KERNEL_GEMM_SIMT 4 /* K2 with the FP32 SIMT GEMM only (the comparator for K2)      */
 #define BC_KERNEL_FUSED 5    /* K3: whole tree per 128-query tile on the tensor cores (tcgen05 3xTF32), messages in
-                                tensor memory; trees of <= 128 columns with domains <= 256 states whose live messages fit the 512
-                                TMEM columns, else BC_ELIMIT */
+                                tensor memory; trees of <= 128 columns with domains <= 256 states (<= 128 below the root) whose
+                                live messages fit the 512 TMEM columns, else BC_ELIMIT */
 
 typedef struct bc_model bc_model;
 
