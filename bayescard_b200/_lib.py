@@ -68,6 +68,11 @@ _SIGS = {
     "bc_marginal_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "bc_expectation_marginal_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int,
                                                 C.c_void_p]),
+    "bc_joint_marginal_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                          C.c_int, C.c_void_p]),
+    "bc_model_specialize_joint": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_char_p]),
+    "bc_model_joint_source": (C.c_int64, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t]),
+    "bc_model_joint_hash": (C.c_uint64, [C.c_void_p, C.c_int, C.c_int]),
     "bc_query_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                  C.c_void_p]),
     "bc_query_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include <atomic>
+#include <map>
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
@@ -18,6 +19,8 @@
 #define BC_SPEC_CTR_SLOTS 256
 #define BC_MARGINAL_VERSION 2   // marginal kernels (bc_marg_*): part of their cache name, independent of BC_CODEGEN_VERSION;
                                 // 2: the kernels apply the fan-out mask
+#define BC_JOINT_VERSION 1      // joint marginal kernels (bc_joint_*): part of their cache name
+#define BC_JOINT_MAX_FFMA 32768 // FMA-pipe instructions per entry above which a pair gets no joint module (it expands)
 
 // One record per node, copied to the device and (by K1) into shared memory.  32 bytes.
 struct BcNodeRec {
@@ -36,7 +39,7 @@ struct BcBitsRec {
     int32_t card;
 };
 
-// Specialised marginal kernels of one target node (spec_jit.cu)
+// Specialised marginal kernels of one target node, or joint marginal kernels of one pair of nodes (spec_jit.cu)
 struct BcMargSlot {
     cudaLibrary_t lib = nullptr;
     cudaKernel_t bits = nullptr, dense = nullptr;
@@ -100,7 +103,8 @@ struct bc_model {
     std::atomic<uint32_t> spec_ctr_next{0};
     // specialised marginal kernels, one slot per target node (empty until the first bc_model_specialize_marginal)
     std::vector<BcMargSlot> marg;
-    std::mutex marg_mu;
+    std::map<std::pair<int, int>, BcMargSlot> joint;   // joint marginal kernels, keyed by the ordered pair (a, b)
+    std::mutex marg_mu;                                // guards marg and joint
     BcK2Plan* k2 = nullptr;
     std::mutex k2_mu;                // guards the lazy construction of k2 (pipe_mu may already be held)
     BcK3Plan* k3 = nullptr;          // fused tensor-core tree kernel: edge schedule, TMEM columns, operand images
@@ -174,4 +178,11 @@ int bc_marg_build(bc_model* m, int target, const char* cache_dir);
 bool bc_marg_attached(bc_model* m, int target);
 int bc_marg_launch(bc_model* m, const void* desc, size_t nq, int fmt, const uint32_t* fan_mask, int target, float* out,
                    cudaStream_t stream);
-void bc_marg_free(bc_model* m);
+void bc_marg_free(bc_model* m);   // unloads the marginal and the joint modules
+// joint marginal kernels: spec_codegen.cc (source, hash; BC_ELIMIT above BC_JOINT_MAX_FFMA) and spec_jit.cu (attach, launch)
+int bc_joint_generate(const bc_model& m, int a, int b, std::string* src);
+uint64_t bc_joint_hash_of(const bc_model& m, int a, int b);
+int bc_joint_build(bc_model* m, int a, int b, const char* cache_dir);
+bool bc_joint_attached(bc_model* m, int a, int b);
+int bc_joint_launch(bc_model* m, const void* desc, size_t nq, int fmt, const uint32_t* fan_mask, int a, int b, float* out,
+                    cudaStream_t stream);

@@ -33,6 +33,9 @@
 //   pi_0 = w_0 * lambda_0 * T_0,   pi_i[c] = w_i[c] * lambda_i[c] * sum_p T_i[c][p] * pi_{i-1}[p],   out = pi_k
 // (lambda_i: product of the messages of a_i's children off the path), again one FMA per non-zero CPT entry.  Both passes
 // apply the fan-out mask (p_fmask) as the spec module does: bit v multiplies w_v by fanouts[v].
+//
+// A third module per (model, ordered pair a, b) answers GROUP BY a, b (bc_joint_generate): out[q][i][j], the marginal's chain
+// down to the two targets' lowest common ancestor, then a loop unrolled over the states of one target (gen_joint_body).
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
@@ -224,13 +227,14 @@ struct Gen {
     // with one FMA-pipe instruction per non-zero T_v[c][p]; returns pi_i, one register per state of v.  A path node with a
     // fan-out vector multiplies each state by fanouts[v][c] under its mask bit (@p mul, or a selp between two immediates at a
     // root without lambda), so a query without that bit computes exactly what the kernel without fan-out does.
-    std::vector<std::string> path_step(int v, int skip, const std::vector<std::string>& prev) {
+    // `skip2`: a second child left out (a joint marginal's lowest common ancestor, whose two children lead to the targets).
+    std::vector<std::string> path_step(int v, int skip, const std::vector<std::string>& prev, int skip2 = -1) {
         const BcNodeRec& nd = m.nodes[v];
         const bool root = v == 0;
         const int card = nd.card, cols = root ? 1 : nd.card_pa;
         std::vector<std::string> lam;
         for (int k : kids[v]) {
-            if (k == skip) continue;
+            if (k == skip || k == skip2) continue;
             std::vector<std::string> mk = message(k);
             if (lam.empty()) lam = mk;
             else
@@ -292,12 +296,62 @@ struct Gen {
         }
         return pi;
     }
+
+    // u_v[c] = w_v[c] * fanouts[v][c] (under the mask bit) * prod(messages of v's children other than `skip`): what a node
+    // strictly below the lowest common ancestor of a joint marginal contributes to every term, one register per state.
+    std::vector<std::string> path_weights(int v, int skip) {
+        const BcNodeRec& nd = m.nodes[v];
+        const int card = nd.card;
+        std::vector<std::string> lam;
+        for (int k : kids[v]) {
+            if (k == skip) continue;
+            std::vector<std::string> mk = message(k);
+            if (lam.empty()) lam = mk;
+            else
+                for (int c = 0; c < card; ++c) line("mul.f32 " + lam[c] + ", " + lam[c] + ", " + mk[c] + ";");
+        }
+        line("// ---- joint path node " + I(v) + ": card " + I(card) + ", parent " + I(nd.parent) +
+             (skip < 0 ? " (target)" : ", next " + I(skip)));
+        const bool fan = nd.fan_off >= 0;
+        const std::string pfb = fan ? fan_pred(v) : std::string();
+        std::vector<std::string> wreg(dense ? ((card + 3) / 4) * 4 : 0), u(card);
+        for (int c = 0; c < card; ++c) {
+            std::string lc = lam.empty() ? std::string() : lam[c];
+            if (fan) {
+                const std::string fv = fhex(m.fan[nd.fan_off + c]);
+                if (lc.empty()) {
+                    lc = F();
+                    line("selp.f32 " + lc + ", " + fv + ", 0f3F800000, " + pfb + ";");
+                } else {
+                    line("@" + pfb + " mul.f32 " + lc + ", " + lc + ", " + fv + ";");
+                }
+            }
+            if (dense) {
+                const int j = c / 4;
+                if (wreg[4 * j].empty()) {
+                    std::string a = F(), b = F(), c2 = F(), d = F();
+                    line("ld.global.nc.v4.f32 {" + a + ", " + b + ", " + c2 + ", " + d + "}, [%rrow+" + I(4LL * (nd.lam_off + 4 * j)) + "];");
+                    wreg[4 * j] = a; wreg[4 * j + 1] = b; wreg[4 * j + 2] = c2; wreg[4 * j + 3] = d;
+                }
+                u[c] = wreg[c];
+                if (!lc.empty()) {
+                    u[c] = F();
+                    line("mul.f32 " + u[c] + ", " + wreg[c] + ", " + lc + ";");
+                }
+            } else {
+                u[c] = F();
+                line("selp.f32 " + u[c] + ", " + (lc.empty() ? std::string("0f3F800000") : lc) + ", 0f00000000, " + bit_pred(v, c) + ";");
+            }
+        }
+        return u;
+    }
 };
 
 // Wraps the straight-line body of `g` in the query loop of one entry point and stores `res`, res.size() consecutive floats
-// per query (row q at out + 4 * res.size() * q).
+// per query (row q at out + 4 * res.size() * q).  With `body_row` > 0 the body stores its own results instead (res is
+// empty): body_row floats per query at [%rtmp + 4 k], under %pvalid; the row address is set before the body.
 std::string gen_entry(const bc_model& m, Gen& g, const char* name, bool dense, int threads, int min_blocks,
-                      const std::vector<std::string>& res) {
+                      const std::vector<std::string>& res, long long body_row = 0) {
     const int sync_every = g.sync_every;
     const int words = m.bits_words;
     const bool dynamic = env_int("BC_SPEC_DYNAMIC", 1) != 0;
@@ -395,12 +449,19 @@ std::string gen_entry(const bc_model& m, Gen& g, const char* name, bool dense, i
             e("@%pfm ld.global.nc.u32 " + g.fmw[w] + ", [%rtmp+" + I(4LL * w) + "];");
         }
     }
+    if (body_row > 0) {
+        if (!clamp) e("setp.lt.u64 %pvalid, %rq, %rnq;");
+        e("mul.lo.u64 %rtmp, %rq, " + I(4LL * body_row) + ";");
+        e("add.u64 %rtmp, %rtmp, %rout;");
+    }
     s += g.out;
-    if (res.size() == 1) e("shl.b64 %rtmp, %rq, 2;");
-    else e("mul.lo.u64 %rtmp, %rq, " + I(4LL * (long long)res.size()) + ";");
-    e("add.u64 %rtmp, %rtmp, %rout;");
-    for (size_t b = 0; b < res.size(); ++b)
-        e(std::string(clamp ? "@%pvalid " : "") + "st.global.f32 [%rtmp" + (b ? "+" + I(4LL * (long long)b) : "") + "], " + res[b] + ";");
+    if (!res.empty()) {
+        if (res.size() == 1) e("shl.b64 %rtmp, %rq, 2;");
+        else e("mul.lo.u64 %rtmp, %rq, " + I(4LL * (long long)res.size()) + ";");
+        e("add.u64 %rtmp, %rtmp, %rout;");
+        for (size_t b = 0; b < res.size(); ++b)
+            e(std::string(clamp ? "@%pvalid " : "") + "st.global.f32 [%rtmp" + (b ? "+" + I(4LL * (long long)b) : "") + "], " + res[b] + ";");
+    }
     if (!dynamic) {
         e("add.u64 %rq, %rq, %rstep;");
         if (sync_every > 0) e("add.u64 %rqb, %rqb, %rstep;");
@@ -455,6 +516,154 @@ std::string gen_marginal_kernel(const bc_model& m, int target, bool dense, int t
     for (size_t i = 0; i < path.size(); ++i) pi = g.path_step(path[i], i + 1 < path.size() ? path[i + 1] : -1, pi);
     if (n_fma) *n_fma = g.n_fma;
     return gen_entry(m, g, dense ? "bc_marg_dense" : "bc_marg_bits", dense, threads, min_blocks, pi);
+}
+
+// The joint marginal of (a, b) with loop node X (a or b; Y is the other), c their lowest common ancestor:
+//   1. every subtree off the root -> X and root -> Y paths upward (Gen::message), the chain root -> c (path_step, c leaving out
+//      both children towards X and Y): pi_c;
+//   2. u_v = w_v * fan_v * (messages of v's off-path children) for every v strictly below c on the X - c - Y path;
+//   3. for each state i of X, unrolled: X below c: row i of T_X times u_X[i], climbed to c (u folded in at each node), times
+//      pi_c; X == c: pi_c[i] times column i of the first CPT towards Y.  Then down to Y as path_step does, with the stored u,
+//      and the card(Y) results of this i are stored at once.
+// A structural zero (no non-zero CPT entry reaches a state) emits nothing and is stored from a zero register.
+struct JointBody {
+    long long n_fma = 0, cost = 0, pipe = 0;   // CPT-carrying FMAs; FMA-pipe + store instructions; FMA-pipe instructions
+    std::string path;
+};
+
+float cpt_at(const bc_model& m, int v, int s, int p) {
+    const BcNodeRec& nd = m.nodes[v];
+    return m.arena[nd.cpt_off + (v == 0 ? s : (int64_t)s * nd.stride + p)];
+}
+
+JointBody gen_joint_body(const bc_model& m, Gen& g, int a, int b, int X, bool dense) {
+    g.sync_every = env_int("BC_SPEC_SYNC_EVERY", 0);
+    if (!dense)
+        for (int w = 0; w < m.bits_words; ++w) g.words.push_back(g.R());
+    if (g.any_fan)
+        for (int w = 0; w < m.mask_words; ++w) g.fmw.push_back(g.R());
+    const int Y = X == a ? b : a;
+    auto root_path = [&](int v) {
+        std::vector<int> p;
+        for (; v > 0; v = m.nodes[v].parent) p.push_back(v);
+        p.push_back(0);
+        std::reverse(p.begin(), p.end());
+        return p;
+    };
+    const std::vector<int> px = root_path(X), py = root_path(Y);
+    size_t d = 0;
+    while (d + 1 < px.size() && d + 1 < py.size() && px[d + 1] == py[d + 1]) ++d;
+    const int c = px[d];
+    const std::vector<int> up(px.begin() + d + 1, px.end());     // c's child towards X ... X (empty: X == c)
+    const std::vector<int> down(py.begin() + d + 1, py.end());   // c's child towards Y ... Y (empty: Y == c)
+    // 1. off the paths
+    std::vector<std::string> pi;
+    for (size_t i = 0; i < d; ++i) pi = g.path_step(px[i], px[i + 1], pi);
+    const int cx = up.empty() ? -1 : up[0], cy = down.empty() ? -1 : down[0];
+    pi = g.path_step(c, cx >= 0 ? cx : cy, pi, cx >= 0 ? cy : -1);
+    const int card_c = m.nodes[c].card;
+    std::vector<char> pz(card_c);   // all-zero CPT rows of c: path_step's shared zero, no mass
+    for (int s = 0; s < card_c; ++s) {
+        bool any = false;
+        for (int p = 0; p < (c == 0 ? 1 : m.nodes[c].card_pa); ++p) any |= cpt_at(m, c, s, p) != 0.f;
+        pz[s] = !any;
+    }
+    // 2. per-node vectors
+    std::vector<std::vector<std::string>> u(m.n);
+    for (size_t k = 0; k < up.size(); ++k) u[up[k]] = g.path_weights(up[k], k + 1 < up.size() ? up[k + 1] : -1);
+    for (size_t k = 0; k < down.size(); ++k) u[down[k]] = g.path_weights(down[k], k + 1 < down.size() ? down[k + 1] : -1);
+    const std::string zero = g.F();
+    g.line("mov.f32 " + zero + ", 0f00000000;");
+    // fma into x (a fresh register on the first term)
+    auto acc = [&](std::string& x, const std::string& r, float t) {
+        ++g.n_fma;
+        if (x.empty()) { x = g.F(); g.line("mul.f32 " + x + ", " + r + ", " + fhex(t) + ";"); }
+        else g.line("fma.rn.f32 " + x + ", " + r + ", " + fhex(t) + ", " + x + ";");
+    };
+    auto scale = [&](const std::string& x, const std::string& y) { g.line("mul.f32 " + x + ", " + x + ", " + y + ";"); };
+    // down[k0..]: r over the states of down[k0]'s parent -> over the states of Y
+    auto descend = [&](std::vector<std::string> r, size_t k0) {
+        for (size_t k = k0; k < down.size(); ++k) {
+            const int v = down[k];
+            std::vector<std::string> nr(m.nodes[v].card);
+            for (int t = 0; t < m.nodes[v].card; ++t) {
+                for (int s = 0; s < m.nodes[v].card_pa; ++s) {
+                    const float T = cpt_at(m, v, t, s);
+                    if (!r[s].empty() && T != 0.f) acc(nr[t], r[s], T);
+                }
+                if (!nr[t].empty()) scale(nr[t], u[v][t]);
+            }
+            r = nr;
+        }
+        return r;
+    };
+    // 3. the unrolled loop over the states of X
+    const int cb = m.nodes[b].card;
+    for (int i = 0; i < m.nodes[X].card; ++i) {
+        g.line("// ---- state " + I(i) + " of node " + I(X));
+        std::vector<std::string> r;
+        if (!up.empty()) {
+            std::vector<std::string> vec(m.nodes[X].card_pa);
+            for (int p = 0; p < m.nodes[X].card_pa; ++p) {
+                const float T = cpt_at(m, X, i, p);
+                if (T != 0.f) acc(vec[p], u[X][i], T);
+            }
+            for (size_t k = up.size() - 1; k-- > 0;) {
+                const int w = up[k];
+                std::vector<std::string> xin(m.nodes[w].card), nv(m.nodes[w].card_pa);
+                for (int s = 0; s < m.nodes[w].card; ++s)
+                    if (!vec[s].empty()) {
+                        xin[s] = g.F();
+                        g.line("mul.f32 " + xin[s] + ", " + vec[s] + ", " + u[w][s] + ";");
+                    }
+                for (int p = 0; p < m.nodes[w].card_pa; ++p)
+                    for (int s = 0; s < m.nodes[w].card; ++s) {
+                        const float T = cpt_at(m, w, s, p);
+                        if (!xin[s].empty() && T != 0.f) acc(nv[p], xin[s], T);
+                    }
+                vec = nv;
+            }
+            r.assign(card_c, std::string());
+            for (int s = 0; s < card_c; ++s)
+                if (!vec[s].empty() && !pz[s]) {
+                    r[s] = g.F();
+                    g.line("mul.f32 " + r[s] + ", " + vec[s] + ", " + pi[s] + ";");
+                }
+            r = descend(r, 0);
+        } else {
+            const int v = down[0];
+            r.assign(m.nodes[v].card, std::string());
+            if (!pz[i])
+                for (int t = 0; t < m.nodes[v].card; ++t) {
+                    const float T = cpt_at(m, v, t, i);
+                    if (T == 0.f) continue;
+                    acc(r[t], pi[i], T);
+                    scale(r[t], u[v][t]);
+                }
+            r = descend(r, 1);
+        }
+        for (int j = 0; j < m.nodes[Y].card; ++j) {
+            const long long idx = X == a ? (long long)i * cb + j : (long long)j * cb + i;
+            g.line("@%pvalid st.global.f32 [%rtmp" + (idx ? "+" + I(4 * idx) : std::string()) + "], " + (r[j].empty() ? zero : r[j]) + ";");
+        }
+    }
+    JointBody jb;
+    jb.n_fma = g.n_fma;
+    for (size_t pos = 0; pos < g.out.size();) {
+        size_t e = g.out.find('\n', pos);
+        if (e == std::string::npos) e = g.out.size();
+        size_t k = g.out.find_first_not_of(' ', pos);
+        if (k < e && g.out[k] == '@') k = g.out.find(' ', k) + 1;
+        auto starts = [&](const char* op) { return g.out.compare(k, std::strlen(op), op) == 0; };
+        if (k < e && (starts("mul.f32") || starts("fma.rn.f32") || starts("add.f32"))) ++jb.pipe;
+        if (k < e && starts("st.global")) ++jb.cost;
+        pos = e + 1;
+    }
+    jb.cost += jb.pipe;
+    for (size_t k = 0; k < px.size(); ++k) jb.path += (k ? " -> " : "") + I(px[k]);
+    jb.path += "  |  ";
+    for (size_t k = d; k < py.size(); ++k) jb.path += (k > d ? " -> " : "") + I(py[k]);
+    return jb;
 }
 
 }  // namespace
@@ -542,6 +751,56 @@ uint64_t bc_marginal_hash_of(const bc_model& m, int target) {
         for (size_t i = 0; i < n; ++i) { h ^= b[i]; h *= 1099511628211ull; }
     };
     const int tag[2] = {BC_MARGINAL_VERSION, target};
+    mix(tag, sizeof(tag));
+    return h;
+}
+
+// Module of the joint marginal of the ordered pair (a, b): bc_joint_bits / bc_joint_dense, the loop, geometry and work counter
+// of the bc_spec_* entries, out[q][i][j] (i < card(a), j < card(b)) stored by the body.  The loop node X is whichever of a, b
+// gives the BITS entry fewer FMA-pipe plus store instructions (a on a tie); both entries use it.  The header's BC_SPEC_FFMA
+// counts the FMA-pipe instructions that carry a CPT entry.  BC_ELIMIT when an entry would hold more than BC_JOINT_MAX_FFMA
+// FMA-pipe instructions: the straight line grows with card(X) times the path's CPTs.
+int bc_joint_generate(const bc_model& m, int a, int b, std::string* src) {
+    int threads, min_blocks;
+    bc_spec_geometry(m, &threads, &min_blocks);
+    Gen ga(m, false), gb(m, false);
+    const JointBody ja = gen_joint_body(m, ga, a, b, a, false), jb = gen_joint_body(m, gb, a, b, b, false);
+    const bool pick_b = jb.cost < ja.cost;
+    Gen& g1 = pick_b ? gb : ga;
+    const JointBody& j1 = pick_b ? jb : ja;
+    const int X = pick_b ? b : a;
+    long long pipe = j1.pipe;
+    Gen g2(m, true);
+    if (pipe <= BC_JOINT_MAX_FFMA) pipe = std::max(pipe, gen_joint_body(m, g2, a, b, X, true).pipe);
+    if (pipe > BC_JOINT_MAX_FFMA) {
+        bc_set_error("joint marginal of nodes %d, %d: %lld FMA-pipe instructions per query, above the cap of %d (BC_JOINT_MAX_FFMA)",
+                     a, b, pipe, BC_JOINT_MAX_FFMA);
+        return BC_ELIMIT;
+    }
+    const long long row = (long long)m.nodes[a].card * m.nodes[b].card;
+    std::string s;
+    s += "//\n// Generated by bayescard_b200 spec_codegen, joint marginal generator (version " + I(BC_JOINT_VERSION) + ", codegen version " +
+         I(BC_CODEGEN_VERSION) + ") -- do not edit.\n";
+    s += "// nodes: " + I(m.n) + "  a: " + I(a) + " (card " + I(m.nodes[a].card) + ")  b: " + I(b) + " (card " + I(m.nodes[b].card) +
+         ")  X: " + I(X) + "  paths: " + j1.path + "\n";
+    s += "// BC_SPEC_THREADS=" + I(threads) + " BC_SPEC_MIN_BLOCKS=" + I(min_blocks) + " BC_SPEC_FFMA=" + I(j1.n_fma) +
+         " FMA-pipe=" + I(j1.pipe) + "\n//\n";
+    s += ".version 8.7\n.target sm_100a\n.address_size 64\n\n";
+    // {threads per CTA, a, b, joint generator version}
+    s += ".visible .global .align 4 .u32 bc_joint_meta[4] = {" + I(threads) + ", " + I(a) + ", " + I(b) + ", " + I(BC_JOINT_VERSION) + "};\n\n";
+    s += gen_entry(m, g1, "bc_joint_bits", false, threads, min_blocks, {}, row);
+    s += gen_entry(m, g2, "bc_joint_dense", true, threads, min_blocks, {}, row);
+    src->swap(s);
+    return BC_OK;
+}
+
+uint64_t bc_joint_hash_of(const bc_model& m, int a, int b) {
+    uint64_t h = bc_spec_hash_of(m);
+    auto mix = [&](const void* p, size_t n) {
+        const unsigned char* c = static_cast<const unsigned char*>(p);
+        for (size_t i = 0; i < n; ++i) { h ^= c[i]; h *= 1099511628211ull; }
+    };
+    const int tag[3] = {BC_JOINT_VERSION, a, b};
     mix(tag, sizeof(tag));
     return h;
 }

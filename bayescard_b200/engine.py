@@ -10,7 +10,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import threading
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -47,6 +47,8 @@ class DeviceModel:
         self.spec_error: Optional[str] = None
         self.marginal_error: Dict[int, str] = {}   # target node -> why its specialised marginal kernel is missing
         self._marginal_built: Dict[int, bool] = {}
+        self.joint_error: Dict[Tuple[int, int], str] = {}   # ordered pair -> why its joint module is missing
+        self._joint_built: Dict[Tuple[int, int], bool] = {}
         self._specialize = specialize and device >= 0   # update() re-specialises under the same policy
         self._cache_dir = cache_dir
         if specialize and device >= 0:
@@ -181,6 +183,88 @@ class DeviceModel:
                                      torch.cuda.current_stream().cuda_stream, d_mask.data_ptr() if d_mask is not None else 0)
             return d_out.cpu().numpy().reshape(n, card)
 
+    # ------------------------------------------------------------------ GROUP BY two columns (joint marginals)
+    def _check_pair(self, a: int, b: int):
+        a, b = self._check_node(a), self._check_node(b)
+        if a == b:
+            raise ValueError(f"a joint marginal needs two distinct nodes, got {a} twice")
+        return a, b
+
+    def specialize_joint(self, a: int, b: int, cache_dir: Optional[str] = None) -> bool:
+        """Attach the joint module of the ordered pair ``(a, b)`` (built on the first call, then kept).  A failure -- such
+        as a pair above the generator's size cap -- is recorded in ``joint_error[(a, b)]`` and not retried;
+        ``run_joint_*`` then serve the pair by expansion."""
+        a, b = self._check_pair(a, b)
+        if (a, b) not in self._joint_built:
+            cache_dir = L.SPEC_CACHE_DIR if cache_dir is None else cache_dir
+            try:
+                L.check(L.lib().bc_model_specialize_joint(self._h, a, b, cache_dir.encode() if cache_dir else None))
+                self._joint_built[(a, b)] = True
+            except L.BayesCardError as e:
+                self.joint_error[(a, b)] = str(e)
+                self._joint_built[(a, b)] = False
+        return self._joint_built[(a, b)]
+
+    def joint_source(self, a: int, b: int) -> str:
+        lib = L.lib()
+        a, b = self._check_pair(a, b)
+        n = lib.bc_model_joint_source(self._h, a, b, None, 0)
+        if n < 0:
+            L.check(int(n))
+        buf = C.create_string_buffer(int(n))
+        lib.bc_model_joint_source(self._h, a, b, buf, int(n))
+        return buf.value.decode()
+
+    def joint_hash(self, a: int, b: int) -> int:
+        a, b = self._check_pair(a, b)
+        return int(L.lib().bc_model_joint_hash(self._h, a, b))
+
+    def run_joint_device(self, desc_ptr: int, n: int, fmt: int, a: int, b: int, out_ptr: int, kernel: int = L.KERNEL_AUTO,
+                         stream: int = 0, mask_ptr: int = 0) -> None:
+        """``bc_joint_marginal_batch`` on DEVICE buffers: ``out`` receives ``[n][card(a)][card(b)]`` fp32; ``mask_ptr``: 0 or
+        ``n * mask_words`` uint32 fan-out mask rows."""
+        L.check(L.lib().bc_joint_marginal_batch(self._h, desc_ptr or None, n, fmt, mask_ptr or None, int(a), int(b), out_ptr or None,
+                                                kernel, stream or None))
+
+    # one call's device output stays below this many bytes (run_joint_host chunks the rows)
+    JOINT_OUT_BYTES = 256 << 20
+
+    def run_joint_host(self, desc: np.ndarray, fmt: int, a: int, b: int, kernel: int = L.KERNEL_AUTO,
+                       mask: Optional[np.ndarray] = None) -> np.ndarray:
+        """BITS / DENSE_F32 rows from the host -> ``ndarray [n, card(a), card(b)]`` fp32: the mass of every pair of states of
+        ``a`` and ``b`` under each row, with the fan-out columns of ``mask`` (``[n, mask_words]`` uint32, or ``None``)
+        multiplied in.  The rows go in chunks whose output is at most ``JOINT_OUT_BYTES`` on the device."""
+        a, b = self._check_pair(a, b)
+        stride = self.desc_stride(fmt)
+        desc = np.ascontiguousarray(desc)
+        n = desc.nbytes // stride
+        if desc.nbytes != n * stride:
+            raise ValueError(f"descriptor buffer of {desc.nbytes} B is not a multiple of the row stride {stride}")
+        if mask is not None:
+            mask = np.ascontiguousarray(mask, dtype=np.uint32).reshape(-1)
+            if mask.size != n * self.mask_words:
+                raise ValueError("fan-out mask has the wrong size")
+        ca, cb = int(self.tm.card[a]), int(self.tm.card[b])
+        out = np.zeros((n, ca, cb), dtype=np.float32)
+        if n == 0 or self.device < 0:   # (the library still validates the arguments)
+            L.check(L.lib().bc_joint_marginal_batch(self._h, None, n, fmt, None, a, b, None, kernel, None))
+            return out
+        import torch
+
+        rows = desc.reshape(-1).view(np.uint8).reshape(n, stride)
+        chunk = max(1, self.JOINT_OUT_BYTES // (4 * ca * cb))
+        dev = torch.device("cuda", self.device)
+        with torch.cuda.device(dev):
+            for q0 in range(0, n, chunk):
+                q1 = min(n, q0 + chunk)
+                d_desc = torch.from_numpy(rows[q0:q1].reshape(-1)).to(dev)
+                d_mask = None if mask is None else torch.from_numpy(mask[q0 * self.mask_words:q1 * self.mask_words]).to(dev)
+                d_out = torch.empty((q1 - q0) * ca * cb, dtype=torch.float32, device=dev)
+                self.run_joint_device(d_desc.data_ptr(), q1 - q0, fmt, a, b, d_out.data_ptr(), kernel,
+                                      torch.cuda.current_stream().cuda_stream, d_mask.data_ptr() if d_mask is not None else 0)
+                out[q0:q1] = d_out.cpu().numpy().reshape(q1 - q0, ca, cb)
+        return out
+
     # ------------------------------------------------------------------ incremental update (DESIGN.md section 9e)
     def attach_counts(self, counts: np.ndarray) -> None:
         """Keep ``counts`` (uint64, ``fit.count_layout`` order) on the device as the counts behind the CPTs
@@ -189,6 +273,8 @@ class DeviceModel:
         L.check(L.lib().bc_model_set_counts(self._h, counts.ctypes.data, counts.size))
         self._marginal_built.clear()
         self.marginal_error.clear()
+        self._joint_built.clear()
+        self.joint_error.clear()
 
     def get_counts(self, node_first: int = 0, node_count: Optional[int] = None) -> np.ndarray:
         """The attached counters of nodes ``[node_first, node_first + node_count)`` (default: to the last node)."""
@@ -264,6 +350,8 @@ class DeviceModel:
         if nodes.size:
             self._marginal_built.clear()
             self.marginal_error.clear()
+            self._joint_built.clear()
+            self.joint_error.clear()
             if self._specialize:
                 try:
                     self.specialize(self._cache_dir)

@@ -90,6 +90,27 @@ class VariableEliminationB200:
             out[d_idx] = dm.run_marginal_host(d_desc, L.DESC_DENSE_F32, v, kernel, None if mask is None else mask[d_idx])
         return out
 
+    def joint_batch(self, decoded, names, kernel: Optional[int] = None,
+                    fanouts: Optional[Sequence[Sequence[str]]] = None) -> np.ndarray:
+        """GROUP BY two columns ``names = (name_a, name_b)``: ``[len(decoded), card_a, card_b]`` fp64, the mass of every pair
+        of states under the already decoded query i, weighted by the fan-out columns ``fanouts[i]`` when given
+        (``bc_joint_marginal_batch``).  The first call for a pair attaches its joint module; a sharded machine answers on
+        its first replica."""
+        a, b = (self.tm._index[n] for n in names)
+        kernel = self.kernel if kernel is None else kernel
+        dm = self._single
+        if self.specialize and kernel in (L.KERNEL_AUTO, L.KERNEL_SPEC) and dm.device >= 0:
+            dm.specialize_joint(a, b)
+        out = np.zeros((len(decoded), int(self.tm.card[a]), int(self.tm.card[b])), dtype=np.float64)
+        if len(decoded) == 0:
+            return out
+        b_idx, b_desc, d_idx, d_desc, mask = self.compiler.pack(decoded, fanouts)
+        if len(b_idx):
+            out[b_idx] = dm.run_joint_host(b_desc, L.DESC_BITS, a, b, kernel, None if mask is None else mask[b_idx])
+        if len(d_idx):
+            out[d_idx] = dm.run_joint_host(d_desc, L.DESC_DENSE_F32, a, b, kernel, None if mask is None else mask[d_idx])
+        return out
+
     @staticmethod
     def _unit(q):
         """``n_distinct`` falsy: the reference sums the selected rows (ExactInference.py:138-139)."""

@@ -13,6 +13,7 @@ forms ``groupby_batch`` / ``expectation_groupby_batch`` (one pass per query for 
 from __future__ import annotations
 
 import copy
+import itertools
 from typing import Any, Dict, List, Optional, Sequence
 
 import numpy as np
@@ -171,8 +172,8 @@ class Bayescard_BN:
             out[dense_idx] = m.dev.run_host(dense_rows, L.DESC_DENSE_F32, None, m.kernel)
         return out if return_prob else out * self.nrows
 
-    # ------------------------------------------------------------------ GROUP BY one column
-    def groupby_batch(self, queries: Sequence[dict], column: str, return_prob: bool = False):
+    # ------------------------------------------------------------------ GROUP BY one or two columns
+    def groupby_batch(self, queries: Sequence[dict], column, return_prob: bool = False):
         """``SELECT column, COUNT(*) ... WHERE P GROUP BY column`` for a batch of predicate dicts ``P``: returns ``(keys,
         est)`` with ``est[i, j]`` the estimate of group ``keys[j]`` under query i -- one pass per query on the GPU
         (``bc_marginal_batch``) instead of one query per group value.
@@ -183,31 +184,34 @@ class Bayescard_BN:
         * A continuous column, or one without an encoding: the keys are the bins (continuous: the bin's interval from
           ``mapping``); the predicate on ``column`` stays, with its coverage weights, and ``est(b) = nrows * M[b]``.
 
+        ``column`` may also be a pair ``(a, b)`` of distinct columns, ``GROUP BY a, b`` (``bc_joint_marginal_batch``, one
+        pass per query for all ``card(a) * card(b)`` groups): the keys are the row-major pairs ``(ka, kb)`` of each column's
+        keys under the rules above, and for two categorical columns ``est(va, vb) = nrows * J[bin(va)][bin(vb)] * weight(va)
+        * weight(vb)``, which is ``self.query({**P_without_a_b, a: va, b: vb})``; ``est`` is ``[n, Ka * Kb]``.
+
         Undecodable queries give a zero row; a query without predicates gives the column's marginal."""
         return self._groupby(queries, None, column, return_prob)
 
-    def expectation_groupby_batch(self, queries: Sequence[dict], fanout_attrs: Sequence[Sequence[str]], column: str,
+    def expectation_groupby_batch(self, queries: Sequence[dict], fanout_attrs: Sequence[Sequence[str]], column,
                                   return_prob: bool = False):
         """:meth:`groupby_batch` of an expectation: query i is weighted by its fan-out columns ``fanout_attrs[i]``, so that
         ``est[i, j]`` is ``self.expectation({**P_without_column, column: keys[j]}, fanout_attrs[i])`` for the values the
         predicate on ``column`` selects (0 for the others) -- the factor of a join estimate for every group at once, one
-        pass per query (``bc_expectation_marginal_batch``).  Keys and value selection are those of :meth:`groupby_batch`.
-        Undecodable queries give a zero row (where ``expectation`` raises ``AttributeError``).  Grouping by a fan-out column
-        raises ``ValueError``."""
-        v = self.tree._index.get(column)
-        if column in self.fanout_attr or (v is not None and self.tree.fan_vector(v) is not None):
-            raise ValueError(f"column {column!r} is a fan-out column; GROUP BY needs a column of the table")
+        pass per query (``bc_expectation_marginal_batch``, or ``bc_joint_marginal_batch`` for a pair of columns).  Keys and
+        value selection are those of :meth:`groupby_batch`.  Undecodable queries give a zero row (where ``expectation``
+        raises ``AttributeError``).  Grouping by a fan-out column raises ``ValueError``."""
         if len(fanout_attrs) != len(queries):
             raise ValueError("one list of fan-out columns per query")
         return self._groupby(queries, [list(f or []) for f in fanout_attrs], column, return_prob)
 
-    def _groupby(self, queries, fanout_attrs, column, return_prob):
-        m = self._machine()
+    def _group_keys(self, m, column):
+        """``(node, categorical, keys, key_bin, key_wt)`` of one grouping column (``key_bin`` / ``key_wt``: categorical only)."""
         v = self.tree._index.get(column)
         if v is None:
             raise ValueError(f"column {column!r} is not a node of this model")
         col = m.compiler.cols[column]
         categorical = col.kind != "continuous" and col.enc is not None
+        key_bin = key_wt = None
         if categorical:
             keys = list(col.pair)
             key_bin = np.asarray([col.pair[k][0] for k in keys], dtype=np.int64)
@@ -216,40 +220,63 @@ class Bayescard_BN:
             keys = [tuple(col.edges[b]) for b in range(int(self.tree.card[v]))]
         else:
             keys = list(range(int(self.tree.card[v])))
+        return v, categorical, keys, key_bin, key_wt
+
+    def _groupby(self, queries, fanout_attrs, column, return_prob):
+        cols = (column,) if isinstance(column, str) else tuple(column)
+        if len(cols) not in (1, 2) or len(set(cols)) != len(cols):
+            raise ValueError(f"GROUP BY takes one column or a pair of distinct columns, got {column!r}")
+        if fanout_attrs is not None or len(cols) == 2:
+            for c in cols:
+                v = self.tree._index.get(c)
+                if c in self.fanout_attr or (v is not None and self.tree.fan_vector(v) is not None):
+                    raise ValueError(f"column {c!r} is a fan-out column; GROUP BY needs a column of the table")
+        m = self._machine()
+        info = [self._group_keys(m, c) for c in cols]
+        keys = info[0][2] if len(cols) == 1 else list(itertools.product(info[0][2], info[1][2]))
         est = np.zeros((len(queries), len(keys)), dtype=np.float64)
         decoded, keep, sel = [], [], []
         for i, q in enumerate(queries):
-            if categorical:
-                s = np.ones(len(keys), dtype=bool)
-                if column in q:
-                    s = m.compiler.select_values(column, q[column])
-                    if s is None:
-                        continue
-                q = {k: x for k, x in q.items() if k != column}
-                sel.append(s)
-            b, w = m.compiler.decode(q)
-            if b is None:
+            s_q = []
+            for c, (_, categorical, ck, _, _) in zip(cols, info):
                 if categorical:
-                    sel.pop()
-                continue
-            decoded.append((b, w))
-            keep.append(i)
-        if decoded:
-            M = m.marginal_batch(decoded, column, fanouts=None if fanout_attrs is None else [fanout_attrs[i] for i in keep])
-            if categorical:
-                est[keep] = M[:, key_bin] * key_wt[None, :] * np.asarray(sel)
+                    s = np.ones(len(ck), dtype=bool)
+                    if c in q:
+                        s = m.compiler.select_values(c, q[c])
+                        if s is None:
+                            break
+                    q = {k: x for k, x in q.items() if k != c}
+                s_q.append(s if categorical else None)
             else:
-                est[keep] = M
+                b, w = m.compiler.decode(q)
+                if b is not None:
+                    decoded.append((b, w))
+                    keep.append(i)
+                    sel.append(s_q)
+        if decoded:
+            fans = None if fanout_attrs is None else [fanout_attrs[i] for i in keep]
+            if len(cols) == 1:
+                M = m.marginal_batch(decoded, cols[0], fanouts=fans)
+            else:
+                M = m.joint_batch(decoded, cols, fanouts=fans)
+            for k, (_, categorical, _, key_bin, key_wt) in enumerate(info):
+                if categorical:
+                    shape = [1] * M.ndim
+                    shape[1 + k] = -1
+                    S = np.asarray([s[k] for s in sel]).reshape([len(sel)] + shape[1:])
+                    M = np.take(M, key_bin, axis=1 + k) * key_wt.reshape(shape) * S
+            est[keep] = M.reshape(len(keep), -1)
         return keys, (est if return_prob else est * self.nrows)
 
-    def groupby(self, query: dict, column: str, return_prob: bool = False) -> Dict[Any, float]:
-        """One query of :meth:`groupby_batch`: ``{key: estimate}``."""
+    def groupby(self, query: dict, column, return_prob: bool = False) -> Dict[Any, float]:
+        """One query of :meth:`groupby_batch` (one column or a pair): ``{key: estimate}``."""
         keys, est = self.groupby_batch([query], column, return_prob)
         return {k: float(e) for k, e in zip(keys, est[0])}
 
     def groupby_sql_batch(self, sqls: Sequence[str], return_prob: bool = False) -> List[Dict[Any, float]]:
-        """``SELECT a, COUNT(*) FROM t [WHERE ...] GROUP BY a`` texts -> one ``{key: estimate}`` per text; the texts that
-        group by the same column are answered in one batch."""
+        """``SELECT a, COUNT(*) FROM t [WHERE ...] GROUP BY a`` and ``SELECT a, b, COUNT(*) ... GROUP BY a, b`` texts -> one
+        ``{key: estimate}`` per text (two columns: keys ``(ka, kb)``); the texts that group by the same columns are answered
+        in one batch."""
         from .sql_front import parse_groupby_single_table
 
         parsed = [parse_groupby_single_table(s, self) for s in sqls]

@@ -1,5 +1,6 @@
 """Single-table SQL front end: ``SELECT COUNT(*) FROM t WHERE a OP v AND ...`` -> predicate dict, and
-``SELECT a, COUNT(*) FROM t [WHERE ...] GROUP BY a`` -> (predicate dict, grouping column).
+``SELECT a, COUNT(*) FROM t [WHERE ...] GROUP BY a`` -> (predicate dict, grouping column), and the same with two grouping
+columns.
 
 Same input language and output as the reference's ``parse_query_single_table``
 (``Evaluation/cardinality_estimation.py:22-119``), which feeds ``Bayescard_BN.query``:
@@ -111,25 +112,28 @@ _GROUPBY = re.compile(r"^\s*SELECT\s+(?P<sel>.+?)\s+FROM\s+(?P<table>\S+?)(?:\s+
                       r"\s+GROUP\s+BY\s+(?P<group>.+?)\s*;?\s*$", re.S | re.I)
 
 
-def parse_groupby_single_table(sql: str, bn) -> Tuple[Dict[str, Any], str]:
-    """``SELECT a, COUNT(*) FROM t [WHERE ...] GROUP BY a`` -> ``(query, "a")``.  The WHERE clause is read as by
-    :func:`parse_query_single_table` (``split_predicate`` / ``add_predicate``).  One grouping column, which the model
-    must hold, and a select list of that column and ``COUNT(*)``; anything else raises ``ValueError``."""
+def parse_groupby_single_table(sql: str, bn):
+    """``SELECT a, COUNT(*) FROM t [WHERE ...] GROUP BY a`` -> ``(query, "a")`` and ``SELECT a, b, COUNT(*) FROM t [WHERE ...]
+    GROUP BY a, b`` -> ``(query, ("a", "b"))``.  The WHERE clause is read as by :func:`parse_query_single_table`
+    (``split_predicate`` / ``add_predicate``).  One or two distinct grouping columns, which the model must hold, and a
+    select list of exactly those columns and ``COUNT(*)``; anything else raises ``ValueError``."""
     mt = _GROUPBY.match(sql)
     if mt is None:
         raise ValueError("not a single-table GROUP BY query: " + sql)
     group = [g.strip() for g in mt.group("group").split(",")]
-    if len(group) != 1 or not group[0]:
-        raise ValueError("GROUP BY takes exactly one column here, got " + mt.group("group"))
-    column = group[0]
-    if column not in bn.attr_type or column not in bn.tree._index:
-        raise ValueError(f"GROUP BY column {column!r} is not a column of the model")
+    if len(group) not in (1, 2) or not all(group):
+        raise ValueError("GROUP BY takes one or two columns here, got " + mt.group("group"))
+    if len(set(group)) != len(group):
+        raise ValueError("GROUP BY names a column twice: " + mt.group("group"))
+    for column in group:
+        if column not in bn.attr_type or column not in bn.tree._index:
+            raise ValueError(f"GROUP BY column {column!r} is not a column of the model")
     sel = sorted(x.strip().replace(" ", "").upper() for x in mt.group("sel").split(","))
-    if sel != sorted(["COUNT(*)", column.upper()]):
-        raise ValueError("the select list must be the grouping column and COUNT(*): " + mt.group("sel"))
+    if sel != sorted(["COUNT(*)"] + [c.upper() for c in group]):
+        raise ValueError("the select list must be the grouping columns and COUNT(*): " + mt.group("sel"))
     out: Dict[str, Any] = {}
     if mt.group("where"):
         for pred in mt.group("where").split(" AND "):
             attr, op, val = split_predicate(pred.strip())
             add_predicate(bn, out, attr, op, val)
-    return out, column
+    return out, (group[0] if len(group) == 1 else tuple(group))

@@ -200,6 +200,31 @@ BC_API int bc_model_specialize_marginal(bc_model* m, int target, const char* cac
 BC_API int64_t bc_model_marginal_source(const bc_model* m, int target, char* buf, size_t buf_bytes);
 BC_API uint64_t bc_model_marginal_hash(const bc_model* m, int target);
 
+/* ---- GROUP BY two columns: per-(state, state) counts of two nodes a != b under each query's predicates ----------------
+ * Replaces `[bn.query({**P, a: va, b: vb}) for va, vb in pairs]` -- card(a) * card(b) full evaluations per query -- with ONE
+ * pass per query.  With bc_expectation_marginal_batch's weights w'_v (fan-out mask bit v multiplies w_v by fanouts[v];
+ * NULL: no mask)
+ *     out[q][i][j] = sum_{x : x_a = i, x_b = j} prod_v w'_v[x_v] T_v[x_v, x_pa(v)]        contiguous fp32 [n][card(a)][card(b)]
+ * Both targets' own weights apply.  Summing over j gives bc_expectation_marginal_batch(a) on the same row and mask, over i
+ * the same for b, over both bc_query_batch.  Rows are BITS or DENSE_F32.  DEVICE pointers, stream ordered.  kernel:
+ *   BC_KERNEL_AUTO   the joint module of (a, b) when it is attached, otherwise the expansion below
+ *   BC_KERNEL_SPEC   the joint module of (a, b); BC_ECOMPILE when it is not attached
+ *   any other id     the expansion: every row becomes card(a) rows (a's weights restricted to one state each, the mask row
+ *                    repeated; chunks of <= 256 MB), evaluated by bc_expectation_marginal_batch(b) with that kernel id
+ * BC_EINVAL for a == b, a node outside [0, n_nodes), a RANGE_* or unknown format, NULL pointers or a host-only model;
+ * n_queries == 0 is BC_OK with no launch.  Results below the fp32 range are not carried. */
+BC_API int bc_joint_marginal_batch(bc_model* m, const void* desc, size_t n_queries, int desc_format, const uint32_t* fanout_mask,
+                                   int a, int b, float* out, int kernel, void* stream);
+/* Build (or load "<cache_dir>/joint_<hash>.cubin") the joint module of the ordered pair (a, b): straight-line sm_100a code
+ * unrolled over the states of one of the two nodes, attached through the driver JIT and kept on the model.  BC_ELIMIT (with
+ * the instruction count and the cap in bc_last_error) for a pair whose body would exceed BC_JOINT_MAX_FFMA = 32768 FMA-pipe
+ * instructions per entry point; AUTO then expands. */
+BC_API int bc_model_specialize_joint(bc_model* m, int a, int b, const char* cache_dir);
+/* Its generated PTX (host-only models too; the bytes needed including the NUL, or BC_ELIMIT as above) and the hash that names
+ * its cache entry (model, ordered pair and joint generator version; 0 for an invalid pair). */
+BC_API int64_t bc_model_joint_source(const bc_model* m, int a, int b, char* buf, size_t buf_bytes);
+BC_API uint64_t bc_model_joint_hash(const bc_model* m, int a, int b);
+
 /* Device-side descriptor conversion (stream ordered, DEVICE pointers): RANGE_U8 / RANGE_U16 -> BITS. */
 BC_API int bc_convert_desc(bc_model* m, const void* src, int src_format, void* dst, int dst_format, size_t n_queries,
                     void* stream);
